@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- PSO train pairs/sec on synthetic SDXL-shaped data (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--pairs B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--pairs B] [--dump-outputs DIR]
 
 Workload (config.workload): the configuration BASELINE.json's metric is quoted on ("SDXL 128x128 latents") = configs[2]'s
 per-GPU slice: SDXL-DMD2 online PSO, LoRA rank 64, 1024x1024 (128x128 latents), bf16 (`--config dmd128`, default); configs[1]
@@ -46,6 +46,8 @@ Numbers on the JSON line:
   turbo64             : a short run of BASELINE configs[1] appended after the main timing (value, ms_per_step, roofline).
   cpu_baseline        : the oracle port of the reference's PyTorch path (fp32, same UNet architecture) on this box's host
                         cores, one micro-step of ONE pair (bounded sample), N = 1 / rank 0 only.
+`--dump-outputs DIR` writes what the last timed step left for its caller as DIR/<name>.npy (see dump_outputs), so that two
+builds can be compared output for output on the same seeded inputs.
 `--impl reference` times that oracle port as the reference arm (the reference is Python that needs diffusers / peft /
 accelerate and /root/reference; none exist on the GPU box -- DESIGN.md).
 """
@@ -68,6 +70,7 @@ if ROOT not in sys.path:
 METRIC = "pso_train_pairs_per_sec"
 UNIT = "pairs/s"
 ACCUM = 6  # gradient_accumulation_steps (2) x trained timesteps (3): turbo trainer :232, dmd2 trainer :236
+DUMP_SAMPLE = 1 << 21  # --dump-outputs: at most 4 x 8 MB of float32 from the flat LoRA buffers
 _COMMON = ("online PSO micro-step (2 policy + 2 frozen-reference UNet forwards, fused PSO loss+grad, backward), random-init "
            "SDXL-architecture UNet (2.57 B params, 560 LoRA projections), bf16, optimizer step every 6 micro-steps")
 # BASELINE.json's metric is quoted on SDXL 128x128 latents = configs[2] (SDXL-DMD2, rank 64, 1024 px): the default.
@@ -316,6 +319,11 @@ class B200Arm:
         lora.set_wgrad_stream(args.wgrad_stream)
         lora.set_in_launch_dependencies(not args.no_inlaunch_deps)
         lora.set_programmatic_launch(args.programmatic_launch)
+        # --deterministic (default): the same arguments compute the same outputs on every run, which is what --dump-outputs
+        # compares -- dA / dB reductions not split over CTAs (one accumulation per element and launch) and the stock torch
+        # kernels of the step on their deterministic algorithms, for the lifetime of this arm (close() restores the defaults)
+        lora.set_deterministic_wgrad(args.deterministic)
+        torch.use_deterministic_algorithms(args.deterministic)
         unet.train()
         if args.grad_checkpointing:
             unet.enable_gradient_checkpointing()  # turbo trainer :358
@@ -438,6 +446,7 @@ class B200Arm:
                 marks[i + 1].record()
             ev1.record()
             self.barrier()
+        self.last_loss = loss
         launches = self.L.psob200_launch_count() - launches0 + K * self.launches_per_micro
         per_step = [marks[i].elapsed_time(marks[i + 1]) for i in range(K)]
         ms_per_step = self.max_over_ranks(ev0.elapsed_time(ev1)) / K
@@ -446,6 +455,23 @@ class B200Arm:
         if K >= self.accum:  # at least one optimizer boundary inside the timed region: its (pre-clip) gradient norm
             out["grad_norm"] = float(self.opt.grad_norm.item())
         return out
+
+    def dump_outputs(self, out_dir):
+        """What the last timed step left for its caller, as float32 .npy files: the loss it returned, the gradient norm of
+        the last optimizer boundary, and the four flat LoRA buffers (adapter parameters, accumulated gradient, both AdamW
+        moments).  A buffer longer than DUMP_SAMPLE elements is stored at DUMP_SAMPLE positions drawn with a fixed seed."""
+        import numpy as np
+        os.makedirs(out_dir, exist_ok=True)
+        bufs = {"lora_params": self.opt.flat_param, "lora_grad": self.bucket.flat, "adamw_exp_avg": self.opt.exp_avg,
+                "adamw_exp_avg_sq": self.opt.exp_avg_sq}
+        n = self.bucket.flat.numel()
+        idx = None
+        if n > DUMP_SAMPLE:
+            idx = torch.randint(0, n, (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values.to(self.dev)
+        out = {"loss": self.last_loss.detach(), "grad_norm": self.opt.grad_norm}
+        out.update({k: (v if idx is None else v[idx]) for k, v in bufs.items()})
+        for k, v in out.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v.float().cpu().numpy())
 
     def e2e(self, K):
         """The same K steps with the step's inputs copied from pinned host memory and the loss read back, every step."""
@@ -598,6 +624,8 @@ class B200Arm:
 
     def close(self):
         self.lora.set_wgrad_stream(False)
+        self.lora.set_deterministic_wgrad(False)
+        torch.use_deterministic_algorithms(False)
         self.graph = self.static_loss = None
         self.unet = self.opt = self.bucket = self.d = self.host = None
         import gc
@@ -778,6 +806,9 @@ def run_b200(args):
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: there is no CPU fallback for the b200 arm")
     L = _lib.lib()  # fail loudly if the CUDA library is missing
+    if args.deterministic:  # what torch's deterministic mode needs before the first cuBLAS call (B200Arm switches the mode)
+        os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")  # 8 x 4 MiB: a fixed cuBLAS workspace per stream
+        torch.utils.deterministic.fill_uninitialized_memory = False  # no NaN fill of every torch.empty: not needed for that
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -790,6 +821,8 @@ def run_b200(args):
     if not args.no_graph:
         arm.capture()
     t = arm.timed(K, W)
+    if args.dump_outputs and rank == 0:
+        arm.dump_outputs(args.dump_outputs)
     e2e = arm.e2e(K)
     peak_hbm_gb = round(torch.cuda.max_memory_allocated(dev) / 2 ** 30, 2)  # before the second (instrumented) graph
     roofline, skinny = arm.instrumented(t["ms_per_step"], peaks)
@@ -1046,12 +1079,21 @@ def parse_args(argv=None):
                          "the printed numbers of such a run are not bench values)")
     ap.add_argument("--no-eager-baseline", action="store_true", help="skip the torch-eager-on-this-GPU baseline")
     ap.add_argument("--no-turbo64", action="store_true", help="skip the short configs[1] block after the main timing")
+    ap.add_argument("--deterministic", action=argparse.BooleanOptionalAction, default=True,
+                    help="this library's arms (headline, turbo64) with unsplit dA / dB reductions and torch's deterministic "
+                         "algorithms: the same arguments give the same outputs (default); --no-deterministic times the library "
+                         "defaults, whose outputs vary from run to run in the last bits (amplified by AdamW). The stock-torch "
+                         "arms always run torch's defaults")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss, gradient norm and (sampled) flat LoRA buffers the last timed step left, as DIR/<name>.npy")
     return ap.parse_args(argv)
 
 
 def main():
     args = parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the b200 arm's outputs; run it without --impl reference")
         run_reference(args)
     else:
         run_b200(args)

@@ -10,8 +10,9 @@ Their only non-torch imports are ``randn_tensor`` and three scheduler class
 names used purely as annotations (turbo :13-15, distilled :13-15); diffusers is
 not installed in this image, so those names are provided by stub modules.
 
-``available()`` is False on the GPU box (no /root/reference there): callers in
-``tests/`` skip, and the committed fixtures under ``tests/golden`` stand in.
+Only the fixture generators ``oracle/make_golden.py`` and ``oracle/make_golden_pins.py``
+run this; ``available()`` says whether the reference is there.  The tests compare with the fixtures under
+``tests/golden`` and need no copy of the reference.
 """
 from __future__ import annotations
 

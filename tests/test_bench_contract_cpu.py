@@ -4,6 +4,10 @@ import json
 import os
 import subprocess
 import sys
+import types
+
+import numpy as np
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -27,3 +31,29 @@ def test_non_zero_ranks_of_the_reference_arm_exit_quietly():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--tiny"],
                          capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_dump_outputs_samples_long_buffers_at_fixed_positions(tmp_path, monkeypatch):
+    """--dump-outputs on buffers longer than DUMP_SAMPLE (the SDXL case): the same seeded positions of every flat buffer, in
+    ascending order, the same on every call; loss and gradient norm as they are."""
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 64)
+    n = 1000
+    flat = torch.arange(n, dtype=torch.float32)
+    opt = types.SimpleNamespace(flat_param=flat, exp_avg=2 * flat, exp_avg_sq=3 * flat, grad_norm=torch.tensor([0.5]))
+    arm = types.SimpleNamespace(opt=opt, bucket=types.SimpleNamespace(flat=-flat), last_loss=torch.tensor(1.25),
+                                dev=torch.device("cpu"))
+    for run in ("a", "b"):
+        bench.B200Arm.dump_outputs(arm, str(tmp_path / run))
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")}
+    assert set(got) == {"loss", "grad_norm", "lora_params", "lora_grad", "adamw_exp_avg", "adamw_exp_avg_sq"}
+    assert all(v.dtype == np.float32 for v in got.values())
+    assert float(got["loss"]) == 1.25 and got["grad_norm"].tolist() == [0.5]
+    pos = got["lora_params"]  # the buffer holds its own index: the dump lists the sampled positions
+    assert pos.shape == (64,) and np.all(np.diff(pos) >= 0) and pos.min() >= 0 and pos.max() < n and len(np.unique(pos)) > 32
+    np.testing.assert_array_equal(got["lora_grad"], -pos)
+    np.testing.assert_array_equal(got["adamw_exp_avg"], 2 * pos)
+    np.testing.assert_array_equal(got["adamw_exp_avg_sq"], 3 * pos)
+    for f in got:
+        np.testing.assert_array_equal(got[f], np.load(tmp_path / "b" / (f + ".npy")))

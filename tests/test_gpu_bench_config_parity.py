@@ -1,7 +1,8 @@
 """Parity of the configuration bench.py actually TIMES (VERDICT r1, weak #1): ``product_micro_step_batched`` (win + lose rows in
 one forward of batch 2B) + the frozen-reference forward on a second stream + the dA / dB launches on the weight-gradient side
-stream + stacked projections (``fuse_attention_projections``, ``fuse_cross_attention_kv``) + the fused GEGLU kernels, captured in
-ONE CUDA graph and replayed, with the fused optimizer boundary
+stream + stacked projections (``fuse_attention_projections``, ``fuse_cross_attention_kv``) + the fused GEGLU kernels + the
+deterministic mode (unsplit dA / dB reductions, torch's deterministic algorithms; part 1), captured in ONE CUDA graph and
+replayed, with the fused optimizer boundary
 (``FusedLoRAOptimizer.step``: clip + AdamW + zero_grad + 16-bit operand refresh) between replays.
 
 1. tiny fixture (BASELINE config 1) against the reference's flow restated on the CPU in fp32 (``oracle_micro_step``: 4
@@ -53,8 +54,9 @@ def _capture(pso, lora, unet, d, sched, ref_stream, **kw):
 
 
 @pytest.mark.parametrize("kind", ["turbo", "dmd"])
-def test_graph_replayed_bench_configuration_vs_oracle_across_an_optimizer_boundary(mods, kind):
+def test_graph_replayed_bench_configuration_vs_oracle_across_an_optimizer_boundary(mods, kind, monkeypatch):
     pso, lora, feed_forward = mods
+    monkeypatch.setenv("CUBLAS_WORKSPACE_CONFIG", ":4096:8")  # what torch's deterministic mode requires of cuBLAS
     r, B = 4, 2
     torch.manual_seed(0)
     cfg = sdxl_unet.tiny_config()
@@ -76,6 +78,8 @@ def test_graph_replayed_bench_configuration_vs_oracle_across_an_optimizer_bounda
     assert lora.fuse_cross_attention_kv(gpu) > 0      # ... and the k / v of all cross-attention layers in one launch per forward
     assert feed_forward.install_fused_geglu(gpu) > 0
     lora.set_wgrad_stream(True)
+    lora.set_deterministic_wgrad(True)  # bench.py's default (--deterministic)
+    torch.use_deterministic_algorithms(True)
     try:
         # lr large enough that one AdamW step moves every adapter element by ~1e-2: replay 2 must see the new operands
         opt = lora.FusedLoRAOptimizer(gpu, lr=1e-2, weight_decay=0.0, max_grad_norm=1e9)
@@ -123,6 +127,8 @@ def test_graph_replayed_bench_configuration_vs_oracle_across_an_optimizer_bounda
         assert losses_seen[0] != losses_seen[1], "the replayed graph did not see the updated adapter operands"
     finally:
         lora.set_wgrad_stream(False)
+        lora.set_deterministic_wgrad(False)
+        torch.use_deterministic_algorithms(False)
 
 
 def test_full_sdxl_fixture_graph_replayed_batched_step_vs_eager_separate_forwards(mods):
