@@ -537,6 +537,62 @@ typedef struct psob200_flat_adamw_args {
 PSOB200_API int psob200_flat_adamw_step(const psob200_flat_adamw_args* args, void* stream);
 
 /*
+ * The same optimizer boundary with bitsandbytes' blockwise 8-bit AdamW state (the Turbo recipe's `use_8bit_adam`:
+ * "AdamW(8bit)" over the LoRA parameters, T:428-448; Dettmers et al. 2022, "8-bit Optimizers via Block-wise Quantization").
+ * Clipping, grad_scale, the overflow skip, found_inf, step_dev, norm_out, workspace, sumsq_parts, zero_grad and the operand
+ * refresh are those of psob200_flat_adamw_step; only the moment storage and the update rule differ.
+ *
+ * 8-bit blocks (blocks8: n_blocks8 pairs {flat offset, length}, 0 < length <= block_size, offset a multiple of 8): block b
+ * keeps one fp32 absmax per moment (absmax1[b], absmax2[b]) and one uint8 code per element and moment, at the element's FLAT
+ * position in code1 / code2 (n bytes each).  map1 (signed, first moment) / map2 (unsigned, second moment): 256 sorted
+ * floats each.  Per element, every operation fp32 and rounded separately (no contraction):
+ *   g  = grad * coef                                  (coef as in psob200_flat_adamw_step)
+ *   m  = map1[c1] * absmax1 ;  v = map2[c2] * absmax2
+ *   m  = m * beta1 + (1 - beta1) * g ;  v = v * beta2 + (1 - beta2) * g * g
+ *   bc1 = (float)(1 - beta1^t), bc2 = (float)sqrt(1 - beta2^t)   (double; t = *step_dev + 1, or `step`)
+ *   p  = p + ((-lr * bc2) / bc1) * (m / (sqrt(v) + eps * bc2)) ;  if weight_decay > 0: p = p * (1 - lr * weight_decay)
+ *   absmax = max |m| (max |v|) over the block ;  x = absmax > 0 ? m / absmax : 0
+ *   code   = number of the 255 midpoints (map[i] + map[i+1]) * 0.5 strictly below x ;
+ *   first moment only: when the sign bit of map1[code] differs from that of m, the code steps one towards m's side.
+ * fp32-class ranges (chunks32: n_chunks32 triples {flat offset, length, compact offset}, 0 < length <= block_size, both
+ * offsets multiples of 8): the same formulas with fp32 m / v at exp_avg32 / exp_avg_sq32 [compact offset + i].
+ * The gradient is zeroed over every block and range, rounded up to whole 8-element groups (at most up to n); flat elements
+ * outside them are not touched.  block_size: 256 (one warp per block) or 2048 (one 256-thread CTA per block), else
+ * PSOB200_ERR_SHAPE.  param, grad, operand, code1, code2, exp_avg32, exp_avg_sq32 16-byte aligned, else PSOB200_ERR_ALIGNMENT.
+ * One update launch (plus the norm launch when the norm is not supplied); deterministic; no allocation, no host sync.
+ */
+typedef struct psob200_flat_adamw8_args {
+  float* param;
+  float* grad;
+  uint8_t* code1;
+  uint8_t* code2;
+  float* absmax1;
+  float* absmax2;
+  const float* map1;
+  const float* map2;
+  const int64_t* blocks8;
+  int64_t n_blocks8;
+  const int64_t* chunks32;
+  int64_t n_chunks32;
+  float* exp_avg32;
+  float* exp_avg_sq32;
+  void* operand;
+  float* norm_out;
+  void* workspace;
+  int64_t n;
+  int64_t step;
+  float lr, beta1, beta2, eps, weight_decay, max_grad_norm, grad_scale;
+  int32_t operand_dtype;
+  int32_t n_sumsq_parts;
+  int32_t block_size;
+  double* sumsq_parts;
+  float* found_inf;
+  long long* step_dev;
+} psob200_flat_adamw8_args;
+
+PSOB200_API int psob200_flat_adamw8_step(const psob200_flat_adamw8_args* args, void* stream);
+
+/*
  * The data-parallel exchange of the training step (DDP's gradient all-reduce behind accelerator.prepare, T:491, sync
  * gate T:858) fused with the norm pass of clip_grad_norm_ (T:859), over NVLink SHARP: ONE launch per rank, no NCCL call.
  * The flat fp32 gradient buffer is symmetric memory (same size on every rank of the group) and grad_multicast is its
@@ -625,7 +681,8 @@ PSOB200_API int psob200_clip_preprocess(const psob200_clip_preprocess_args* args
  * verify their mirror of this header: which = 0 schedule, 1 online_pso_args,
  * 2 dreambooth_args, 3 step_args, 4 step_bwd_args, 5 gemm_args,
  * 6 lora_linear_args, 7 flat_adamw_args, 8 geglu_args,
- * 9 flat_allreduce_args, 10 clip_preprocess_args, 11 lora_group_args.  Returns 0 for unknown ids. */
+ * 9 flat_allreduce_args, 10 clip_preprocess_args, 11 lora_group_args,
+ * 12 flat_adamw8_args.  Returns 0 for unknown ids. */
 PSOB200_API size_t psob200_struct_size(int which);
 
 #ifdef __cplusplus

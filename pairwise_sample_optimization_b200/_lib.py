@@ -110,6 +110,16 @@ class FlatAdamwArgs(C.Structure):
                 ("found_inf", _fp), ("step_dev", _vp)]
 
 
+class FlatAdamw8Args(C.Structure):
+    _fields_ = [("param", _fp), ("grad", _fp), ("code1", _vp), ("code2", _vp), ("absmax1", _fp), ("absmax2", _fp),
+                ("map1", _fp), ("map2", _fp), ("blocks8", _vp), ("n_blocks8", C.c_int64), ("chunks32", _vp),
+                ("n_chunks32", C.c_int64), ("exp_avg32", _fp), ("exp_avg_sq32", _fp), ("operand", _vp), ("norm_out", _fp),
+                ("workspace", _vp), ("n", C.c_int64), ("step", C.c_int64), ("lr", C.c_float), ("beta1", C.c_float),
+                ("beta2", C.c_float), ("eps", C.c_float), ("weight_decay", C.c_float), ("max_grad_norm", C.c_float),
+                ("grad_scale", C.c_float), ("operand_dtype", C.c_int32), ("n_sumsq_parts", C.c_int32),
+                ("block_size", C.c_int32), ("sumsq_parts", _vp), ("found_inf", _fp), ("step_dev", _vp)]
+
+
 class FlatAllreduceArgs(C.Structure):
     _fields_ = [("grad_multicast", _vp), ("sumsq_multicast", _vp), ("n", C.c_int64), ("rank", C.c_int32),
                 ("world", C.c_int32), ("scale", C.c_float)]
@@ -130,7 +140,8 @@ class ClipPreprocessArgs(C.Structure):
 
 
 _STRUCTS = {0: Schedule, 1: OnlinePsoArgs, 2: DreamboothArgs, 3: StepArgs, 4: StepBwdArgs, 5: GemmArgs,
-            6: LoraLinearArgs, 7: FlatAdamwArgs, 8: GegluArgs, 9: FlatAllreduceArgs, 10: ClipPreprocessArgs, 11: LoraGroupArgs}
+            6: LoraLinearArgs, 7: FlatAdamwArgs, 8: GegluArgs, 9: FlatAllreduceArgs, 10: ClipPreprocessArgs, 11: LoraGroupArgs,
+            12: FlatAdamw8Args}
 
 # name -> (restype, argtypes): every symbol include/psob200.h declares
 SIGNATURES = {
@@ -154,6 +165,7 @@ SIGNATURES = {
     "psob200_lora_group_forward": (C.c_int, [C.POINTER(LoraGroupArgs), _vp]),
     "psob200_lora_group_backward": (C.c_int, [C.POINTER(LoraGroupArgs), _vp]),
     "psob200_flat_adamw_step": (C.c_int, [C.POINTER(FlatAdamwArgs), _vp]),
+    "psob200_flat_adamw8_step": (C.c_int, [C.POINTER(FlatAdamw8Args), _vp]),
     "psob200_flat_allreduce_sumsq": (C.c_int, [C.POINTER(FlatAllreduceArgs), _vp]),
     "psob200_geglu_forward": (C.c_int, [C.POINTER(GegluArgs), _vp]),
     "psob200_geglu_backward": (C.c_int, [C.POINTER(GegluArgs), _vp]),

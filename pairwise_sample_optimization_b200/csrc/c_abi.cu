@@ -56,6 +56,7 @@ extern "C" size_t psob200_struct_size(int which) {
     case 9: return sizeof(psob200_flat_allreduce_args);
     case 10: return sizeof(psob200_clip_preprocess_args);
     case 11: return sizeof(psob200_lora_group_args);
+    case 12: return sizeof(psob200_flat_adamw8_args);
     default: return 0;
   }
 }

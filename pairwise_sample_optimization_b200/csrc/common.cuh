@@ -258,6 +258,9 @@ inline int consume_launch_error(const char* where, cudaError_t e) {
   return PSOB200_ERR_LAUNCH;
 }
 
+// Launches flat_sumsq_kernel (flat_optimizer.cu): the gradient's sum of squares into ws[0], shared by both AdamW boundaries.
+int launch_flat_sumsq(const float* g, long long n, double* ws, int n_sm, cudaStream_t st);
+
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 inline size_t dtype_size(int32_t dt) { return dt == PSOB200_F32 ? 4 : 2; }
 inline bool valid_dtype(int32_t dt) { return dt == PSOB200_F32 || dt == PSOB200_BF16 || dt == PSOB200_F16; }

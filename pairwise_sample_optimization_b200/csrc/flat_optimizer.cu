@@ -140,6 +140,13 @@ flat_adamw_kernel(float* __restrict__ p, float* __restrict__ g, float* __restric
   }
 }
 
+int launch_flat_sumsq(const float* g, long long n, double* ws, int n_sm, cudaStream_t st) {
+  long long blocks = (n + kOptThreads * 4 - 1) / (kOptThreads * 4);
+  if (blocks > n_sm * 8) blocks = n_sm * 8;
+  flat_sumsq_kernel<<<(unsigned)blocks, kOptThreads, 0, st>>>(g, n, ws);
+  return consume_launch_error("launch flat_sumsq_kernel", cudaSuccess);
+}
+
 }  // namespace psob200
 
 using namespace psob200;
@@ -160,13 +167,10 @@ extern "C" int psob200_flat_adamw_step(const psob200_flat_adamw_args* args, void
     if (n_sm <= 0) n_sm = 148;
     sms.store(n_sm, std::memory_order_relaxed);
   }
-  long long blocks = (o.n + kOptThreads * 4 - 1) / (kOptThreads * 4);
-  if (blocks > n_sm * 8) blocks = n_sm * 8;
   double* ws = reinterpret_cast<double*>(o.workspace);
   if (o.n_sumsq_parts < 0 || (o.n_sumsq_parts > 0 && !o.sumsq_parts)) return PSOB200_ERR_INVALID_ARG;
   if (o.n_sumsq_parts == 0 && (o.max_grad_norm > 0.f || o.norm_out != nullptr)) {
-    flat_sumsq_kernel<<<(unsigned)blocks, kOptThreads, 0, st>>>(o.grad, o.n, ws);
-    const int rc = consume_launch_error("launch flat_sumsq_kernel", cudaSuccess);
+    const int rc = launch_flat_sumsq(o.grad, o.n, ws, n_sm, st);
     if (rc != PSOB200_OK) return rc;
   }
   AdamParams a;
@@ -177,7 +181,7 @@ extern "C" int psob200_flat_adamw_step(const psob200_flat_adamw_args* args, void
   a.grad_scale = o.grad_scale;
   a.found_inf = o.found_inf;
   a.step_dev = o.step_dev;
-  blocks = (o.n + kOptThreads - 1) / kOptThreads;
+  long long blocks = (o.n + kOptThreads - 1) / kOptThreads;
   if (blocks > n_sm * 8) blocks = n_sm * 8;
   if (o.operand == nullptr || o.operand_dtype == PSOB200_BF16)
     flat_adamw_kernel<__nv_bfloat16><<<(unsigned)blocks, kOptThreads, 0, st>>>(

@@ -900,16 +900,74 @@ class SymmetricGradExchange:
         self.handle.barrier(channel=1)  # every slice (and every norm slot) has landed everywhere
 
 
+def dynamic_quant_map(signed: bool) -> torch.Tensor:
+    """bitsandbytes' ``create_dynamic_map(signed, max_exponent_bits=7, total_bits=8)``: the 256 sorted fp32 code values of
+    the 8-bit optimizer state (signed for the first moment, unsigned for the second).  Decade i = 0..6 contributes the
+    means of neighbouring points of ``linspace(0.1, 1, k)`` (k = 2^i + 1 signed, 2^(i+1) + 1 unsigned) times 10^(i-6), and
+    their negatives when signed; then 0 and 1."""
+    data = []
+    for i in range(7):
+        b = torch.linspace(0.1, 1, 2 ** i + 1 if signed else 2 ** (i + 1) + 1)
+        means = (b[:-1] + b[1:]) / 2.0
+        data += ((10 ** (i - 6)) * means).tolist()
+        if signed:
+            data += (-(10 ** (i - 6)) * means).tolist()
+    data += [0.0, 1.0]
+    return torch.tensor(sorted(data), dtype=torch.float32)
+
+
+def blockwise_layout(numels, offsets, block_size: int = 256, min_8bit_size: int = 4096):
+    """Block tables of the 8-bit optimizer state over a flat layout (bitsandbytes' per-tensor blocks): every matrix with
+    ``numel >= min_8bit_size`` is cut into blocks of ``block_size`` elements from its own flat offset (the last one may be
+    short) -> ``blocks8`` int64 [B, 2] = {flat offset, length}; smaller matrices keep fp32 moments in a compact buffer and
+    are cut the same way -> ``chunks32`` int64 [C, 3] = {flat offset, length, compact offset}.  Returns
+    ``(blocks8, chunks32, compact_numel)``; compact offsets are multiples of 8 like the flat ones."""
+    blocks, chunks, compact = [], [], 0
+    for n, off in zip(numels, offsets):
+        if off % 8:
+            raise ValueError(f"flat offset {off} is not a multiple of 8 elements")
+        if n >= min_8bit_size:
+            blocks += [(off + s, min(block_size, n - s)) for s in range(0, n, block_size)]
+        else:
+            chunks += [(off + s, min(block_size, n - s), compact + s) for s in range(0, n, block_size)]
+            compact += (n + 7) // 8 * 8
+    return (torch.tensor(blocks, dtype=torch.int64).reshape(-1, 2), torch.tensor(chunks, dtype=torch.int64).reshape(-1, 3),
+            compact)
+
+
+def _table_positions(table: torch.Tensor):
+    """(row of each covered element, its position at column 0 + i, at column 2 + i if present) of a block / chunk table."""
+    lens = table[:, 1]
+    starts = torch.cumsum(lens, 0) - lens
+    row = torch.repeat_interleave(torch.arange(table.shape[0], device=table.device), lens)
+    i = torch.arange(int(lens.sum()), device=table.device) - starts[row]
+    return row, table[row, 0] + i, (table[row, 2] + i if table.shape[1] > 2 else None)
+
+
+_STATE8 = ("flat_param", "code1", "code2", "absmax1", "absmax2", "exp_avg32", "exp_avg_sq32", "qmap1", "qmap2")
+
+
 class FusedLoRAOptimizer:
     """The optimizer boundary of the training step on the flat LoRA buffers: ``clip_grad_norm_`` + AdamW +
     ``zero_grad`` + refresh of the 16-bit GEMM operands in two kernel launches (psob200_flat_adamw_step) instead of the
     reference's per-parameter kernels (train_online_pso_sdxl_turbo.py:428-448 optimizer, :859 clipping, :860-861
     step / zero_grad).  Parameters, gradients and both Adam moments of every adapter matrix are slices of four flat
     fp32 buffers with one layout; ``self.bucket`` is the gradient buffer (``all_reduce()`` = the data-parallel exchange).
-    Update rule = ``torch.optim.AdamW`` (decoupled weight decay, bias correction)."""
+    Update rule = ``torch.optim.AdamW`` (decoupled weight decay, bias correction).
+
+    ``optim_bits=8`` is the Turbo recipe's ``use_8bit_adam`` (bitsandbytes ``AdamW(optim_bits=8)``, same keyword names):
+    blockwise 8-bit moments (``block_size`` elements per fp32 absmax; matrices below ``min_8bit_size`` elements keep fp32
+    moments), bitsandbytes' update rule (weight decay after the step), one update launch of psob200_flat_adamw8_step.
+    ``exp_avg`` / ``exp_avg_sq`` are then None; ``dequantized_moments()`` gives flat fp32 copies."""
 
     def __init__(self, model: nn.Module, lr: float = 1e-5, betas=(0.9, 0.999), eps: float = 1e-8,
-                 weight_decay: float = 1e-4, max_grad_norm: float = 1.0, exchange: Optional[SymmetricGradExchange] = None):
+                 weight_decay: float = 1e-4, max_grad_norm: float = 1.0, exchange: Optional[SymmetricGradExchange] = None,
+                 optim_bits: int = 32, block_size: int = 256, min_8bit_size: int = 4096):
+        if optim_bits not in (8, 32):
+            raise ValueError(f"optim_bits must be 8 or 32, got {optim_bits}")
+        if optim_bits == 8 and block_size not in (256, 2048):
+            raise ValueError(f"block_size must be 256 or 2048, got {block_size}")
+        self.optim_bits, self.block_size, self.min_8bit_size = optim_bits, block_size, min_8bit_size
         self.exchange = exchange  # None: all_reduce() is one NCCL call; else the fused NVLink-multicast kernel
         self.layers = lora_layers(model)
         self.groups = projection_groups(model)
@@ -921,8 +979,22 @@ class FusedLoRAOptimizer:
         self._parts_ready = False
         flat = self.bucket.flat
         self.flat_param = torch.zeros_like(flat)
-        self.exp_avg = torch.zeros_like(flat)
-        self.exp_avg_sq = torch.zeros_like(flat)
+        if optim_bits == 32:
+            self.exp_avg = torch.zeros_like(flat)
+            self.exp_avg_sq = torch.zeros_like(flat)
+        else:
+            self.exp_avg = self.exp_avg_sq = None
+            blocks8, chunks32, n32 = blockwise_layout([p.numel() for p in self.bucket.params], self.bucket.offsets,
+                                                      block_size, min_8bit_size)
+            dev = flat.device
+            self.blocks8, self.chunks32 = blocks8.to(dev), chunks32.to(dev)
+            self.qmap1, self.qmap2 = dynamic_quant_map(True).to(dev), dynamic_quant_map(False).to(dev)
+            self.code1 = torch.full((flat.numel(),), 127, dtype=torch.uint8, device=dev)  # qmap1[127] == 0
+            self.code2 = torch.zeros(flat.numel(), dtype=torch.uint8, device=dev)         # qmap2[0] == 0
+            self.absmax1 = torch.zeros(blocks8.shape[0], dtype=torch.float32, device=dev)
+            self.absmax2 = torch.zeros_like(self.absmax1)
+            self.exp_avg32 = torch.zeros(n32, dtype=torch.float32, device=dev)
+            self.exp_avg_sq32 = torch.zeros_like(self.exp_avg32)
         op_dtype = self.layers[0].base_layer.weight.dtype
         self.flat_operand = torch.zeros(flat.numel(), dtype=op_dtype, device=flat.device)
         self.workspace = torch.zeros(2, dtype=torch.float64, device=flat.device)
@@ -964,21 +1036,53 @@ class FusedLoRAOptimizer:
     def step(self) -> torch.Tensor:
         """Clip, update, zero the gradient, refresh the operands.  Returns the (pre-clip) gradient norm, on the device."""
         self.step_count += 1
-        a = _lib.FlatAdamwArgs()
+        a = self._launch_args()
+        if self._parts_ready:  # the fused exchange already produced the sum of squares, one piece per rank
+            a.n_sumsq_parts, a.sumsq_parts = self.exchange.world, self.exchange.sumsq_parts_ptr
+            self._parts_ready = False
+        entry = "psob200_flat_adamw_step" if self.optim_bits == 32 else "psob200_flat_adamw8_step"
+        _lib.launch(self.flat_param.device, entry, C.byref(a), _lib.current_stream(self.flat_param.device))
+        self._refresh_unbacked()
+        return self.grad_norm
+
+    def _launch_args(self):
+        """The argument struct of this optimizer's boundary entry point for the next ``step()`` (norm computed in-launch)."""
+        if self.optim_bits == 32:
+            a = _lib.FlatAdamwArgs()
+            a.exp_avg, a.exp_avg_sq = self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr()
+        else:
+            a = _lib.FlatAdamw8Args()
+            a.code1, a.code2 = self.code1.data_ptr(), self.code2.data_ptr()
+            a.absmax1, a.absmax2 = self.absmax1.data_ptr(), self.absmax2.data_ptr()
+            a.map1, a.map2 = self.qmap1.data_ptr(), self.qmap2.data_ptr()
+            a.blocks8, a.n_blocks8 = self.blocks8.data_ptr(), self.blocks8.shape[0]
+            a.chunks32, a.n_chunks32 = self.chunks32.data_ptr(), self.chunks32.shape[0]
+            a.exp_avg32, a.exp_avg_sq32 = self.exp_avg32.data_ptr(), self.exp_avg_sq32.data_ptr()
+            a.block_size = self.block_size
         a.param, a.grad = self.flat_param.data_ptr(), self.bucket.flat.data_ptr()
-        a.exp_avg, a.exp_avg_sq = self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr()
         a.operand, a.operand_dtype = self.flat_operand.data_ptr(), _lib.dtype_code(self.flat_operand)
         a.norm_out, a.workspace = self.grad_norm.data_ptr(), self.workspace.data_ptr()
         a.n, a.step = self.flat_param.numel(), self.step_count
         a.lr, a.beta1, a.beta2, a.eps = self.lr, self.betas[0], self.betas[1], self.eps
         a.weight_decay, a.max_grad_norm, a.grad_scale = self.weight_decay, self.max_grad_norm, float(self.grad_scale)
         a.found_inf, a.step_dev = self.found_inf.data_ptr(), self.step_dev.data_ptr()
-        if self._parts_ready:  # the fused exchange already produced the sum of squares, one piece per rank
-            a.n_sumsq_parts, a.sumsq_parts = self.exchange.world, self.exchange.sumsq_parts_ptr
-            self._parts_ready = False
-        _lib.launch(self.flat_param.device, "psob200_flat_adamw_step", C.byref(a), _lib.current_stream(self.flat_param.device))
-        self._refresh_unbacked()
-        return self.grad_norm
+        return a
+
+    def dequantized_moments(self) -> tuple[torch.Tensor, torch.Tensor]:
+        """Flat fp32 copies of both Adam moments in the parameter layout (8-bit blocks dequantised as the kernel does:
+        ``qmap[code] * absmax``), for inspection and tests.  Elements outside every matrix are 0."""
+        if self.optim_bits == 32:
+            return self.exp_avg.clone(), self.exp_avg_sq.clone()
+        m = torch.zeros_like(self.flat_param)
+        v = torch.zeros_like(self.flat_param)
+        if self.blocks8.shape[0]:
+            blk, pos, _ = _table_positions(self.blocks8)
+            m[pos] = self.qmap1[self.code1[pos].long()] * self.absmax1[blk]
+            v[pos] = self.qmap2[self.code2[pos].long()] * self.absmax2[blk]
+        if self.chunks32.shape[0]:
+            _, pos, cpos = _table_positions(self.chunks32)
+            m[pos], v[pos] = self.exp_avg32[cpos], self.exp_avg_sq32[cpos]
+        return m, v
 
     def _refresh_unbacked(self) -> None:
         for lay, which, dt in self._unbacked:  # padded-pitch copies: re-made in place by the layer itself
@@ -999,17 +1103,33 @@ class FusedLoRAOptimizer:
     # ---- checkpoint / resume (accelerator.save_state / load_state, turbo :889: the AdamW moments and step count travel too)
     def state_dict(self) -> dict:
         """Everything a resumed run needs for bit-identical continuation: the fp32 master parameters, both Adam moments,
-        the count of applied updates (one host sync) and the hyper-parameters.  Tensors are clones on the optimizer's device."""
-        return {"flat_param": self.flat_param.clone(), "exp_avg": self.exp_avg.clone(), "exp_avg_sq": self.exp_avg_sq.clone(),
-                "step": int(self.step_dev.item()), "step_calls": int(self.step_count),
-                "hyper": {"lr": self.lr, "beta1": self.betas[0], "beta2": self.betas[1], "eps": self.eps,
-                          "weight_decay": self.weight_decay, "max_grad_norm": self.max_grad_norm},
-                "layout": {"numel": int(self.flat_param.numel()), "offsets": [int(o) for o in self.bucket.offsets],
-                           "shapes": [list(p.shape) for p in self.bucket.params]}}
+        the count of applied updates (one host sync) and the hyper-parameters.  Tensors are clones on the optimizer's device.
+        With ``optim_bits=8`` the moments are the 8-bit state instead (codes, absmax, compact fp32 moments, both maps) and
+        the dict also records ``optim_bits``, ``block_size`` and ``min_8bit_size``."""
+        if self.optim_bits == 32:
+            sd = {"flat_param": self.flat_param.clone(), "exp_avg": self.exp_avg.clone(), "exp_avg_sq": self.exp_avg_sq.clone()}
+        else:
+            sd = {k: getattr(self, k).clone() for k in _STATE8}
+        sd.update({"step": int(self.step_dev.item()), "step_calls": int(self.step_count),
+                   "hyper": {"lr": self.lr, "beta1": self.betas[0], "beta2": self.betas[1], "eps": self.eps,
+                             "weight_decay": self.weight_decay, "max_grad_norm": self.max_grad_norm},
+                   "layout": {"numel": int(self.flat_param.numel()), "offsets": [int(o) for o in self.bucket.offsets],
+                              "shapes": [list(p.shape) for p in self.bucket.params]}})
+        if self.optim_bits == 8:
+            sd.update({"optim_bits": 8, "block_size": self.block_size, "min_8bit_size": self.min_8bit_size})
+        return sd
 
     def load_state_dict(self, sd: dict, load_hyper: bool = True) -> None:
         """Inverse of ``state_dict()``.  The parameters live in ``flat_param`` (every adapter ``weight`` is a view of it), so
         loading also restores the adapters; the 16-bit operand copies the GEMM kernels read are refreshed; the gradient is zeroed."""
+        bits = int(sd.get("optim_bits", 32))
+        if bits != self.optim_bits:
+            raise _lib.Psob200Error(f"optimizer state was saved with optim_bits={bits}; this optimizer has optim_bits="
+                                    f"{self.optim_bits} (the moments of the two modes are stored differently)")
+        if bits == 8 and (int(sd["block_size"]) != self.block_size or int(sd["min_8bit_size"]) != self.min_8bit_size):
+            raise _lib.Psob200Error(f"8-bit optimizer state was saved with block_size={sd['block_size']}, min_8bit_size="
+                                    f"{sd['min_8bit_size']}; this optimizer has block_size={self.block_size}, "
+                                    f"min_8bit_size={self.min_8bit_size}")
         lay = sd["layout"]
         if lay["numel"] != self.flat_param.numel() or list(lay["offsets"]) != [int(o) for o in self.bucket.offsets] or \
                 [list(x) for x in lay["shapes"]] != [list(p.shape) for p in self.bucket.params]:
@@ -1017,10 +1137,16 @@ class FusedLoRAOptimizer:
                                     "fuse_attention_projections / fuse_cross_attention_kv were not called the same way before "
                                     "the optimizer was built (lora_parameters() orders the buffers by group and bank)")
         dev = self.flat_param.device
+        if bits == 8 and not (torch.equal(sd["qmap1"].cpu(), self.qmap1.cpu()) and torch.equal(sd["qmap2"].cpu(), self.qmap2.cpu())):
+            raise _lib.Psob200Error("8-bit optimizer state was saved with other quantisation maps")
         with torch.no_grad():
-            self.flat_param.copy_(sd["flat_param"].to(dev))
-            self.exp_avg.copy_(sd["exp_avg"].to(dev))
-            self.exp_avg_sq.copy_(sd["exp_avg_sq"].to(dev))
+            if bits == 32:
+                self.flat_param.copy_(sd["flat_param"].to(dev))
+                self.exp_avg.copy_(sd["exp_avg"].to(dev))
+                self.exp_avg_sq.copy_(sd["exp_avg_sq"].to(dev))
+            else:
+                for k in _STATE8:
+                    getattr(self, k).copy_(sd[k].to(dev))
             self.step_dev.fill_(int(sd["step"]))
             self.flat_operand.copy_(self.flat_param)  # what psob200_flat_adamw_step would have left
         self.step_count = int(sd.get("step_calls", sd["step"]))
