@@ -19,7 +19,7 @@ import os
 
 import torch
 
-from .lora import _STATE8, LoRALinear
+from .lora import LoRALinear
 
 WEIGHT_NAME = "pytorch_lora_weights.safetensors"
 OPTIMIZER_NAME = "optimizer.safetensors"  # accelerate writes optimizer.bin next to the model files (save_state, turbo :889)
@@ -98,19 +98,15 @@ def load_lora_weights(path: str, unet: torch.nn.Module, strict: bool = True) -> 
 def save_optimizer_state(save_directory: str, optimizer, name: str = OPTIMIZER_NAME) -> str:
     """The resumable part of ``accelerator.save_state`` (turbo :886-889) for ``lora.FusedLoRAOptimizer``: fp32 master
     parameters, both AdamW moments, the count of applied updates and the hyper-parameters, in one safetensors file.
-    With ``optim_bits=8`` the moments are the 8-bit state (uint8 codes, absmax arrays, compact fp32 moments, both maps) and
-    the metadata also records ``optim_bits``, ``block_size`` and ``min_8bit_size``."""
+    Every tensor of ``optimizer.state_dict()`` is stored as a tensor and every other entry as JSON metadata, so the 8-bit
+    state (uint8 codes, absmax arrays, compact fp32 moments, both maps, and the keys that describe its format) travels
+    the same way."""
     import json
     from safetensors.torch import save_file
     os.makedirs(save_directory, exist_ok=True)
     sd = optimizer.state_dict()
-    eight = sd.get("optim_bits", 32) == 8
-    names = _STATE8 if eight else ("flat_param", "exp_avg", "exp_avg_sq")
-    tensors = {k: sd[k].to("cpu").contiguous() for k in names}
-    meta = {"format": "pt", "step": str(sd["step"]), "step_calls": str(sd["step_calls"]), "hyper": json.dumps(sd["hyper"]),
-            "layout": json.dumps(sd["layout"])}
-    if eight:
-        meta.update({k: str(sd[k]) for k in ("optim_bits", "block_size", "min_8bit_size")})
+    tensors = {k: v.to("cpu").contiguous() for k, v in sd.items() if isinstance(v, torch.Tensor)}
+    meta = {"format": "pt", **{k: json.dumps(v) for k, v in sd.items() if not isinstance(v, torch.Tensor)}}
     path = os.path.join(save_directory, name)
     save_file(tensors, path, metadata=meta)
     return path
@@ -126,11 +122,7 @@ def load_optimizer_state(path: str, optimizer, load_hyper: bool = True) -> None:
     with safe_open(path, framework="pt", device="cpu") as f:
         meta = f.metadata()
         sd = {k: f.get_tensor(k) for k in f.keys()}
-    for k in ("optim_bits", "block_size", "min_8bit_size"):  # absent from 32-bit files
-        if k in meta:
-            sd[k] = int(meta[k])
-    sd["step"], sd["step_calls"] = int(meta["step"]), int(meta["step_calls"])
-    sd["hyper"], sd["layout"] = json.loads(meta["hyper"]), json.loads(meta["layout"])
+    sd.update({k: json.loads(v) for k, v in meta.items() if k != "format"})
     optimizer.load_state_dict(sd, load_hyper=load_hyper)
 
 

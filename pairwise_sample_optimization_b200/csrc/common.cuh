@@ -35,6 +35,21 @@ struct PerDevice {  // static storage: zero-initialised
   std::atomic<T>& here() { return v[device_slot()]; }
 };
 
+// SM count of the current device for grid sizing, queried once per device (148, a B200's, when the query fails).
+inline int sm_count() {
+  static PerDevice<int> per_device;
+  std::atomic<int>& cached = per_device.here();
+  int v = cached.load(std::memory_order_relaxed);
+  if (v > 0) return v;
+  int dev = 0, n = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
+    cudaGetLastError();
+    return 148;
+  }
+  cached.store(n, std::memory_order_relaxed);
+  return n;
+}
+
 // ---------------------------------------------------------------------------------------------
 // 8-element (one "chunk") vector access.  bf16/fp16: one 128-bit transaction; fp32: two.
 // Loads are streaming (read once): non-coherent path, no L1 allocation.
@@ -257,9 +272,6 @@ inline int consume_launch_error(const char* where, cudaError_t e) {
   cudaGetLastError();
   return PSOB200_ERR_LAUNCH;
 }
-
-// Launches flat_sumsq_kernel (flat_optimizer.cu): the gradient's sum of squares into ws[0], shared by both AdamW boundaries.
-int launch_flat_sumsq(const float* g, long long n, double* ws, int n_sm, cudaStream_t st);
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 inline size_t dtype_size(int32_t dt) { return dt == PSOB200_F32 ? 4 : 2; }

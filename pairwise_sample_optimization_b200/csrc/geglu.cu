@@ -180,8 +180,7 @@ static int geglu_check(const psob200_geglu_args& a, bool bwd) {
 template <typename Kernel>
 static dim3 geglu_grid(const psob200_geglu_args& a, Kernel kernel) {
   const long long bx = (a.I + kGegluColThreads * 8 - 1) / (kGegluColThreads * 8);
-  int sms = psob200_device_sm_count();
-  if (sms <= 0) sms = 148;
+  const int sms = sm_count();
   static PerDevice<int> cached_dev;  // per kernel instantiation (this function is a template) and device: queried once
   std::atomic<int>& cached = cached_dev.here();
   int per_sm = cached.load(std::memory_order_relaxed);

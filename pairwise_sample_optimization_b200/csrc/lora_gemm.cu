@@ -631,20 +631,6 @@ static int env_fused_bn() {
   return env;
 }
 
-static int gemm_sm_count() {
-  static PerDevice<int> per_device;
-  std::atomic<int>& cached = per_device.here();
-  int v = cached.load(std::memory_order_relaxed);
-  if (v > 0) return v;
-  int dev = 0, n = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
-    cudaGetLastError();
-    return 148;
-  }
-  cached.store(n, std::memory_order_relaxed);
-  return n;
-}
-
 // per-tile fixed cost of the pair kernel in units of one accumulator column: measured per-wave times at K = 1344 are
 // 6.7 us (bn 128) and 9.7 us (bn 256) = 3.7 us + 23.4 ns per column (tools/diag_lora_parts.py --bn ...)
 constexpr int kTileFixedCols = 160;
@@ -709,7 +695,7 @@ struct MapKey { const void* p; long long rows, cols, ld; int box; };
 
 static int launch_problems(const HostLaunch& H, cudaStream_t stream) {
   if (H.n_prob < 1 || H.n_prob > kMaxProb) return PSOB200_ERR_INVALID_ARG;
-  const int sms = gemm_sm_count();
+  const int sms = sm_count();
   bool any_dep = false, any_dt = false, any_bias = false, bias_other = false, all_d = true;
   for (int i = 0; i < H.n_prob; ++i) {
     const HostProblem& hp = H.prob[i];

@@ -457,20 +457,6 @@ static int launch_pair(PairKernelArgs ka, bool has_ref, int32_t pred_dtype, int3
   });
 }
 
-static int cached_sm_count() {
-  static PerDevice<int> per_device;
-  std::atomic<int>& cached = per_device.here();
-  int v = cached.load(std::memory_order_relaxed);
-  if (v > 0) return v;
-  int dev = 0, n = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
-    cudaGetLastError();
-    return 148;
-  }
-  cached.store(n, std::memory_order_relaxed);
-  return n;
-}
-
 }  // namespace psob200
 
 using namespace psob200;
@@ -524,7 +510,7 @@ extern "C" int psob200_online_pso_loss_grad(const psob200_schedule* sched, const
   ka.log_lo = (1.0 - eps > 0.0) ? std::log(1.0 - eps) : -HUGE_VAL;  // exp(d) > 0 >= 1-eps: never clamped from below
   ka.log_hi = std::log1p(eps);
   return launch_pair(ka, true, p.pred_dtype, p.latent_dtype, vec_ok, p.tune_threads, p.tune_cluster,
-                     cached_sm_count(), reinterpret_cast<cudaStream_t>(stream));
+                     sm_count(), reinterpret_cast<cudaStream_t>(stream));
 }
 
 extern "C" int psob200_dreambooth_pso_loss_grad(const psob200_dreambooth_args* args, void* stream) {
@@ -561,5 +547,5 @@ extern "C" int psob200_dreambooth_pso_loss_grad(const psob200_dreambooth_args* a
   ka.mode = has_ref ? kModeDbPso : kModeDbPsoDb;
   ka.beta = p.beta_pso; ka.nu = p.neg_defactor; ka.lam = p.prior_loss_weight; ka.loss_scale = p.loss_scale;
   return launch_pair(ka, has_ref, p.pred_dtype, p.latent_dtype, vec_ok, p.tune_threads, p.tune_cluster,
-                     cached_sm_count(), reinterpret_cast<cudaStream_t>(stream));
+                     sm_count(), reinterpret_cast<cudaStream_t>(stream));
 }

@@ -173,6 +173,20 @@ class LoRALinear(nn.Module):
             hit[0] = p._version
         return hit[2]
 
+    def install_operand(self, which: str, dtype: torch.dtype, op: torch.Tensor) -> None:
+        """Use ``op`` (the parameter's shape, row pitch a multiple of 16 bytes) as the 16-bit copy of adapter matrix
+        ``which``: a view of a flat operand buffer that whoever updates the parameter in place keeps current."""
+        p = (self.lora_A if which == "a" else self.lora_B)[self.active_adapter].weight
+        self._op_cache[(which, dtype)] = [p._version, p.data_ptr(), op]
+
+    def refresh_operand(self, which: str, dtype: torch.dtype) -> None:
+        """Re-make the 16-bit copy of adapter matrix ``which`` even though the parameter's version did not change (a kernel
+        wrote the parameter in place)."""
+        hit = self._op_cache.get((which, dtype))
+        if hit is not None:
+            hit[0] = -1
+        self._operand(which, dtype)
+
     def refresh_operands(self) -> None:
         """Bring the 16-bit operand copies up to date with the parameters (call after an optimizer step when the
         forward is replayed from a CUDA graph, where this Python code does not run)."""
@@ -324,6 +338,14 @@ class LoRAProjectionGroup:
         dtype = self.layers[0].base_layer.weight.dtype
         self.stacked_operand("a", dtype)
         self.stacked_operand("b", dtype)
+
+    def refresh_private_operands(self) -> None:
+        """Re-stack the private copies, if the group keeps any, even though no member's version changed (a kernel wrote
+        the parameters in place)."""
+        if self._op:
+            for hit in self._op.values():
+                hit[0] = None
+            self.refresh_operands()
 
     def stacked_grad(self, which: str) -> torch.Tensor:
         """fp32 accumulation target [G r, K] / [G N, r]: the members' slices of the flat bucket when they are adjacent, else
@@ -944,9 +966,6 @@ def _table_positions(table: torch.Tensor):
     return row, table[row, 0] + i, (table[row, 2] + i if table.shape[1] > 2 else None)
 
 
-_STATE8 = ("flat_param", "code1", "code2", "absmax1", "absmax2", "exp_avg32", "exp_avg_sq32", "qmap1", "qmap2")
-
-
 class FusedLoRAOptimizer:
     """The optimizer boundary of the training step on the flat LoRA buffers: ``clip_grad_norm_`` + AdamW +
     ``zero_grad`` + refresh of the 16-bit GEMM operands in two kernel launches (psob200_flat_adamw_step) instead of the
@@ -979,10 +998,15 @@ class FusedLoRAOptimizer:
         self._parts_ready = False
         flat = self.bucket.flat
         self.flat_param = torch.zeros_like(flat)
+        # what state_dict() carries: the state tensors (attribute names) and the keys that describe their format
         if optim_bits == 32:
+            self._state_names, self._format = ("flat_param", "exp_avg", "exp_avg_sq"), {}
             self.exp_avg = torch.zeros_like(flat)
             self.exp_avg_sq = torch.zeros_like(flat)
         else:
+            self._state_names = ("flat_param", "code1", "code2", "absmax1", "absmax2", "exp_avg32", "exp_avg_sq32", "qmap1",
+                                 "qmap2")
+            self._format = {"optim_bits": 8, "block_size": block_size, "min_8bit_size": min_8bit_size}
             self.exp_avg = self.exp_avg_sq = None
             blocks8, chunks32, n32 = blockwise_layout([p.numel() for p in self.bucket.params], self.bucket.offsets,
                                                       block_size, min_8bit_size)
@@ -1020,7 +1044,7 @@ class FusedLoRAOptimizer:
             if p.shape[1] % 8 == 0:
                 op = self.flat_operand[off:off + p.numel()].view(p.shape)
                 op.copy_(view)
-                lay._op_cache[(which, op_dtype)] = [p._version, p.data_ptr(), op]  # kept current by the fused kernel
+                lay.install_operand(which, op_dtype, op)  # kept current by the fused kernel
             else:
                 self._unbacked.append((lay, which, op_dtype))
 
@@ -1036,22 +1060,21 @@ class FusedLoRAOptimizer:
     def step(self) -> torch.Tensor:
         """Clip, update, zero the gradient, refresh the operands.  Returns the (pre-clip) gradient norm, on the device."""
         self.step_count += 1
-        a = self._launch_args()
+        entry, a = self._launch_args()
         if self._parts_ready:  # the fused exchange already produced the sum of squares, one piece per rank
             a.n_sumsq_parts, a.sumsq_parts = self.exchange.world, self.exchange.sumsq_parts_ptr
             self._parts_ready = False
-        entry = "psob200_flat_adamw_step" if self.optim_bits == 32 else "psob200_flat_adamw8_step"
         _lib.launch(self.flat_param.device, entry, C.byref(a), _lib.current_stream(self.flat_param.device))
         self._refresh_unbacked()
         return self.grad_norm
 
     def _launch_args(self):
-        """The argument struct of this optimizer's boundary entry point for the next ``step()`` (norm computed in-launch)."""
+        """``(entry point, argument struct)`` of this optimizer's boundary for the next ``step()`` (norm computed in-launch)."""
         if self.optim_bits == 32:
-            a = _lib.FlatAdamwArgs()
+            entry, a = "psob200_flat_adamw_step", _lib.FlatAdamwArgs()
             a.exp_avg, a.exp_avg_sq = self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr()
         else:
-            a = _lib.FlatAdamw8Args()
+            entry, a = "psob200_flat_adamw8_step", _lib.FlatAdamw8Args()
             a.code1, a.code2 = self.code1.data_ptr(), self.code2.data_ptr()
             a.absmax1, a.absmax2 = self.absmax1.data_ptr(), self.absmax2.data_ptr()
             a.map1, a.map2 = self.qmap1.data_ptr(), self.qmap2.data_ptr()
@@ -1066,7 +1089,7 @@ class FusedLoRAOptimizer:
         a.lr, a.beta1, a.beta2, a.eps = self.lr, self.betas[0], self.betas[1], self.eps
         a.weight_decay, a.max_grad_norm, a.grad_scale = self.weight_decay, self.max_grad_norm, float(self.grad_scale)
         a.found_inf, a.step_dev = self.found_inf.data_ptr(), self.step_dev.data_ptr()
-        return a
+        return entry, a
 
     def dequantized_moments(self) -> tuple[torch.Tensor, torch.Tensor]:
         """Flat fp32 copies of both Adam moments in the parameter layout (8-bit blocks dequantised as the kernel does:
@@ -1086,15 +1109,9 @@ class FusedLoRAOptimizer:
 
     def _refresh_unbacked(self) -> None:
         for lay, which, dt in self._unbacked:  # padded-pitch copies: re-made in place by the layer itself
-            hit = lay._op_cache.get((which, dt))
-            if hit is not None:
-                hit[0] = -1
-            lay._operand(which, dt)
+            lay.refresh_operand(which, dt)
         for g in self.groups:  # stacked groups that keep private (padded) operand copies: re-stacked in place
-            if g.has_private_operands():
-                for hit in g._op.values():
-                    hit[0] = None
-                g.refresh_operands()
+            g.refresh_private_operands()
 
     def zero_grad(self, set_to_none: bool = False) -> None:
         """In-place zero of the flat gradient (``step()`` already leaves it zeroed); ``param.grad`` stays a bucket view."""
@@ -1106,30 +1123,25 @@ class FusedLoRAOptimizer:
         the count of applied updates (one host sync) and the hyper-parameters.  Tensors are clones on the optimizer's device.
         With ``optim_bits=8`` the moments are the 8-bit state instead (codes, absmax, compact fp32 moments, both maps) and
         the dict also records ``optim_bits``, ``block_size`` and ``min_8bit_size``."""
-        if self.optim_bits == 32:
-            sd = {"flat_param": self.flat_param.clone(), "exp_avg": self.exp_avg.clone(), "exp_avg_sq": self.exp_avg_sq.clone()}
-        else:
-            sd = {k: getattr(self, k).clone() for k in _STATE8}
+        sd = {k: getattr(self, k).clone() for k in self._state_names}
         sd.update({"step": int(self.step_dev.item()), "step_calls": int(self.step_count),
                    "hyper": {"lr": self.lr, "beta1": self.betas[0], "beta2": self.betas[1], "eps": self.eps,
                              "weight_decay": self.weight_decay, "max_grad_norm": self.max_grad_norm},
                    "layout": {"numel": int(self.flat_param.numel()), "offsets": [int(o) for o in self.bucket.offsets],
                               "shapes": [list(p.shape) for p in self.bucket.params]}})
-        if self.optim_bits == 8:
-            sd.update({"optim_bits": 8, "block_size": self.block_size, "min_8bit_size": self.min_8bit_size})
+        sd.update(self._format)
         return sd
 
     def load_state_dict(self, sd: dict, load_hyper: bool = True) -> None:
         """Inverse of ``state_dict()``.  The parameters live in ``flat_param`` (every adapter ``weight`` is a view of it), so
         loading also restores the adapters; the 16-bit operand copies the GEMM kernels read are refreshed; the gradient is zeroed."""
-        bits = int(sd.get("optim_bits", 32))
+        bits = int(sd.get("optim_bits", 32))  # fp32 state records no format keys
         if bits != self.optim_bits:
             raise _lib.Psob200Error(f"optimizer state was saved with optim_bits={bits}; this optimizer has optim_bits="
                                     f"{self.optim_bits} (the moments of the two modes are stored differently)")
-        if bits == 8 and (int(sd["block_size"]) != self.block_size or int(sd["min_8bit_size"]) != self.min_8bit_size):
-            raise _lib.Psob200Error(f"8-bit optimizer state was saved with block_size={sd['block_size']}, min_8bit_size="
-                                    f"{sd['min_8bit_size']}; this optimizer has block_size={self.block_size}, "
-                                    f"min_8bit_size={self.min_8bit_size}")
+        if any(int(sd[k]) != v for k, v in self._format.items()):
+            raise _lib.Psob200Error("8-bit optimizer state was saved with " + ", ".join(f"{k}={sd[k]}" for k in self._format)
+                                    + "; this optimizer has " + ", ".join(f"{k}={v}" for k, v in self._format.items()))
         lay = sd["layout"]
         if lay["numel"] != self.flat_param.numel() or list(lay["offsets"]) != [int(o) for o in self.bucket.offsets] or \
                 [list(x) for x in lay["shapes"]] != [list(p.shape) for p in self.bucket.params]:
@@ -1140,13 +1152,8 @@ class FusedLoRAOptimizer:
         if bits == 8 and not (torch.equal(sd["qmap1"].cpu(), self.qmap1.cpu()) and torch.equal(sd["qmap2"].cpu(), self.qmap2.cpu())):
             raise _lib.Psob200Error("8-bit optimizer state was saved with other quantisation maps")
         with torch.no_grad():
-            if bits == 32:
-                self.flat_param.copy_(sd["flat_param"].to(dev))
-                self.exp_avg.copy_(sd["exp_avg"].to(dev))
-                self.exp_avg_sq.copy_(sd["exp_avg_sq"].to(dev))
-            else:
-                for k in _STATE8:
-                    getattr(self, k).copy_(sd[k].to(dev))
+            for k in self._state_names:
+                getattr(self, k).copy_(sd[k].to(dev))
             self.step_dev.fill_(int(sd["step"]))
             self.flat_operand.copy_(self.flat_param)  # what psob200_flat_adamw_step would have left
         self.step_count = int(sd.get("step_calls", sd["step"]))

@@ -45,7 +45,6 @@ def build(shapes, r, bits, dev):
 
 
 def time_boundary(opt, norm, iters, warmup, dev):
-    entry = "psob200_flat_adamw_step" if opt.optim_bits == 32 else "psob200_flat_adamw8_step"
     parts = torch.zeros(1, dtype=torch.float64, device=dev)
     grads = [torch.randn(opt.bucket.flat.numel(), device=dev, generator=torch.Generator(device=dev).manual_seed(s)) * 1e-3
              for s in range(2)]
@@ -53,7 +52,7 @@ def time_boundary(opt, norm, iters, warmup, dev):
     times = []
     for i in range(warmup + iters):
         opt.bucket.flat.copy_(grads[i % 2])
-        a = opt._launch_args()
+        entry, a = opt._launch_args()
         if norm == "supplied":
             parts.fill_(1e-2)
             a.n_sumsq_parts, a.sumsq_parts = 1, parts.data_ptr()
