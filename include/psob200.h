@@ -166,6 +166,34 @@ PSOB200_API int psob200_online_pso_loss_grad(const psob200_schedule* sched, cons
                                  void* stream);
 
 /*
+ * Dynamic loss scaling on the device: the state of torch's GradScaler, which accelerate wraps around every step of the
+ * fp16 recipes (mixed_precision="fp16", T:126; scaler.scale(loss).backward() T:857, unscale_ + clip_grad_norm_ T:859,
+ * scaler.step + scaler.update() T:860).  scale (S) and growth_tracker are DEVICE scalars; nothing reads them on the host.
+ *   loss entry points (*_loss_grad_scaled): the per-pair gradient multiplier is multiplied by *scale before the
+ *     elementwise pass, so grad = S * d loss / d pred is rounded to the prediction dtype once, already scaled; loss and
+ *     stats stay unscaled.  Only `scale` is read.
+ *   optimizer entry points (psob200_flat_adamw*_step_scaled): the unscale factor is (float)(1 / (double)*scale) times
+ *     grad_scale (fp32), used where grad_scale is used without a scaler; the norm is always computed; the last block
+ *     updates S and growth_tracker as torch._amp_update_scale_ does, with found_inf = "the norm is not finite":
+ *       found_inf:  S = (float)(S * backoff_factor), tracker = 0
+ *       else:       t = tracker + 1; t == growth_interval ? (S' = (float)(S * growth_factor), S = S' if finite, tracker = 0)
+ *                                                         : tracker = t          (products in double)
+ *     growth_factor > 1, 0 < backoff_factor < 1, growth_interval > 0, else PSOB200_ERR_INVALID_ARG.
+ */
+typedef struct psob200_loss_scaler {
+  float* scale;            /* device float[1] */
+  int32_t* growth_tracker; /* device int32[1]; unused by the loss entry points (may be NULL there) */
+  double growth_factor;
+  double backoff_factor;
+  int32_t growth_interval;
+  int32_t reserved;
+} psob200_loss_scaler;
+
+/* psob200_online_pso_loss_grad with the gradient scaled by the device loss scale (T:857 under GradScaler). */
+PSOB200_API int psob200_online_pso_loss_grad_scaled(const psob200_schedule* sched, const psob200_online_pso_args* args,
+                                                    const psob200_loss_scaler* scaler, void* stream);
+
+/*
  * Fused DreamBooth-PSO loss + gradient: replaces P:1847-1865 (EDM-style epsilon
  * preconditioning, non-EDM scheduler) + P:1881-1935 + the autograd backward (P:1953).
  * model_pred/ref_pred: raw UNet outputs [2b,N] (`pred_dtype`), rows [0,b) = win images,
@@ -206,6 +234,9 @@ typedef struct psob200_dreambooth_args {
 } psob200_dreambooth_args;
 
 PSOB200_API int psob200_dreambooth_pso_loss_grad(const psob200_dreambooth_args* args, void* stream);
+/* psob200_dreambooth_pso_loss_grad with the gradient scaled by the device loss scale (P:1953 under GradScaler). */
+PSOB200_API int psob200_dreambooth_pso_loss_grad_scaled(const psob200_dreambooth_args* args,
+                                                        const psob200_loss_scaler* scaler, void* stream);
 
 /* ------------------------------------------------------------------------------------
  * One scheduler update + Gaussian log-prob: the body of turbo_step_with_logprob
@@ -535,6 +566,9 @@ typedef struct psob200_flat_adamw_args {
 } psob200_flat_adamw_args;
 
 PSOB200_API int psob200_flat_adamw_step(const psob200_flat_adamw_args* args, void* stream);
+/* psob200_flat_adamw_step unscaled by, and updating, a device loss scaler (GradScaler unscale_ / step / update, T:859-860). */
+PSOB200_API int psob200_flat_adamw_step_scaled(const psob200_flat_adamw_args* args, const psob200_loss_scaler* scaler,
+                                               void* stream);
 
 /*
  * The same optimizer boundary with bitsandbytes' blockwise 8-bit AdamW state (the Turbo recipe's `use_8bit_adam`:
@@ -591,6 +625,9 @@ typedef struct psob200_flat_adamw8_args {
 } psob200_flat_adamw8_args;
 
 PSOB200_API int psob200_flat_adamw8_step(const psob200_flat_adamw8_args* args, void* stream);
+/* psob200_flat_adamw8_step unscaled by, and updating, a device loss scaler (GradScaler around the 8-bit AdamW, T:859-860). */
+PSOB200_API int psob200_flat_adamw8_step_scaled(const psob200_flat_adamw8_args* args, const psob200_loss_scaler* scaler,
+                                                void* stream);
 
 /*
  * The data-parallel exchange of the training step (DDP's gradient all-reduce behind accelerator.prepare, T:491, sync
@@ -682,7 +719,7 @@ PSOB200_API int psob200_clip_preprocess(const psob200_clip_preprocess_args* args
  * 2 dreambooth_args, 3 step_args, 4 step_bwd_args, 5 gemm_args,
  * 6 lora_linear_args, 7 flat_adamw_args, 8 geglu_args,
  * 9 flat_allreduce_args, 10 clip_preprocess_args, 11 lora_group_args,
- * 12 flat_adamw8_args.  Returns 0 for unknown ids. */
+ * 12 flat_adamw8_args, 13 loss_scaler.  Returns 0 for unknown ids. */
 PSOB200_API size_t psob200_struct_size(int which);
 
 #ifdef __cplusplus

@@ -10,10 +10,12 @@ Only what the path needs (SURVEY.md section 8):
 * ``checkpoint``                  LoRA adapters in the reference's safetensors wire format (+ optimizer state)
 * ``reward_preprocess``           decoded images -> CLIP / PickScore ``pixel_values`` on the device (Pillow-exact resize)
 * ``runtime``                     device-resident schedule tables, workspace, status word
+* ``amp``                         fp16 dynamic loss scaling with the scale on the device (GradScaler semantics)
 
 There is no CPU or PyTorch fallback: every op raises if the CUDA library is missing.
 """
-from . import _lib, checkpoint, feed_forward, gemm, lora, reward_preprocess, runtime
+from . import _lib, amp, checkpoint, feed_forward, gemm, lora, reward_preprocess, runtime
+from .amp import DeviceGradScaler
 from .losses import compare, edm_sigmas, pso_db_loss, pso_pair_loss, sample_compare
 from .pso_pytorch.diffusers_patch import (
     _get_x0_from_noise,
@@ -39,4 +41,5 @@ __all__ = [
     "check_status",
     "clip_image_preprocess",
     "DeviceCLIPImageProcessor",
+    "DeviceGradScaler",
 ]

@@ -120,6 +120,11 @@ class FlatAdamw8Args(C.Structure):
                 ("block_size", C.c_int32), ("sumsq_parts", _vp), ("found_inf", _fp), ("step_dev", _vp)]
 
 
+class LossScaler(C.Structure):
+    _fields_ = [("scale", _fp), ("growth_tracker", _ip), ("growth_factor", C.c_double), ("backoff_factor", C.c_double),
+                ("growth_interval", C.c_int32), ("reserved", C.c_int32)]
+
+
 class FlatAllreduceArgs(C.Structure):
     _fields_ = [("grad_multicast", _vp), ("sumsq_multicast", _vp), ("n", C.c_int64), ("rank", C.c_int32),
                 ("world", C.c_int32), ("scale", C.c_float)]
@@ -141,7 +146,7 @@ class ClipPreprocessArgs(C.Structure):
 
 _STRUCTS = {0: Schedule, 1: OnlinePsoArgs, 2: DreamboothArgs, 3: StepArgs, 4: StepBwdArgs, 5: GemmArgs,
             6: LoraLinearArgs, 7: FlatAdamwArgs, 8: GegluArgs, 9: FlatAllreduceArgs, 10: ClipPreprocessArgs, 11: LoraGroupArgs,
-            12: FlatAdamw8Args}
+            12: FlatAdamw8Args, 13: LossScaler}
 
 # name -> (restype, argtypes): every symbol include/psob200.h declares
 SIGNATURES = {
@@ -154,6 +159,9 @@ SIGNATURES = {
     "psob200_pair_loss_workspace_bytes": (C.c_size_t, [C.c_int64]),
     "psob200_online_pso_loss_grad": (C.c_int, [C.POINTER(Schedule), C.POINTER(OnlinePsoArgs), _vp]),
     "psob200_dreambooth_pso_loss_grad": (C.c_int, [C.POINTER(DreamboothArgs), _vp]),
+    "psob200_online_pso_loss_grad_scaled": (C.c_int, [C.POINTER(Schedule), C.POINTER(OnlinePsoArgs), C.POINTER(LossScaler),
+                                                      _vp]),
+    "psob200_dreambooth_pso_loss_grad_scaled": (C.c_int, [C.POINTER(DreamboothArgs), C.POINTER(LossScaler), _vp]),
     "psob200_step_logprob": (C.c_int, [C.POINTER(Schedule), C.POINTER(StepArgs), _vp]),
     "psob200_step_logprob_backward": (C.c_int, [C.POINTER(Schedule), C.POINTER(StepBwdArgs), _vp]),
     "psob200_dmd_x0_from_noise": (C.c_int, [_fp, C.c_int32, _vp, _vp, _vp, C.c_int32, C.c_int64, _vp, C.c_int64,
@@ -166,6 +174,8 @@ SIGNATURES = {
     "psob200_lora_group_backward": (C.c_int, [C.POINTER(LoraGroupArgs), _vp]),
     "psob200_flat_adamw_step": (C.c_int, [C.POINTER(FlatAdamwArgs), _vp]),
     "psob200_flat_adamw8_step": (C.c_int, [C.POINTER(FlatAdamw8Args), _vp]),
+    "psob200_flat_adamw_step_scaled": (C.c_int, [C.POINTER(FlatAdamwArgs), C.POINTER(LossScaler), _vp]),
+    "psob200_flat_adamw8_step_scaled": (C.c_int, [C.POINTER(FlatAdamw8Args), C.POINTER(LossScaler), _vp]),
     "psob200_flat_allreduce_sumsq": (C.c_int, [C.POINTER(FlatAllreduceArgs), _vp]),
     "psob200_geglu_forward": (C.c_int, [C.POINTER(GegluArgs), _vp]),
     "psob200_geglu_backward": (C.c_int, [C.POINTER(GegluArgs), _vp]),

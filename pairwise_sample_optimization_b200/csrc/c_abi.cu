@@ -57,6 +57,7 @@ extern "C" size_t psob200_struct_size(int which) {
     case 10: return sizeof(psob200_clip_preprocess_args);
     case 11: return sizeof(psob200_lora_group_args);
     case 12: return sizeof(psob200_flat_adamw8_args);
+    case 13: return sizeof(psob200_loss_scaler);
     default: return 0;
   }
 }

@@ -92,6 +92,11 @@ struct BoundaryParams {
   double* ws;  // {sum of squares, ticket}
   double* parts;
   int n_parts;
+  // device loss scaler (psob200_loss_scaler; amp_scale NULL = none): unscaled by in the prologue, updated in the epilogue
+  float* amp_scale;
+  int* amp_tracker;
+  double amp_growth, amp_backoff;
+  int amp_interval;
 };
 
 struct BoundaryScalars {
@@ -104,11 +109,14 @@ __device__ __forceinline__ BoundaryScalars boundary_prologue(const BoundaryParam
   // global-norm clip coefficient (accelerate / torch clip_grad_norm_: coef = min(1, max_norm / (norm + 1e-6)))
   double sumsq = a.ws[0];
   for (int r = 0; r < a.n_parts; ++r) sumsq += a.parts[r];  // per-rank slices of the fused exchange (same order on every rank)
-  const float norm = (float)sqrt(sumsq) * a.grad_scale;
+  // unscale factor: with a device loss scaler torch's scale.double().reciprocal().float(), times grad_scale in fp32
+  float grad_scale = a.grad_scale;
+  if (a.amp_scale != nullptr) grad_scale = (float)(1.0 / (double)*a.amp_scale) * grad_scale;
+  const float norm = (float)sqrt(sumsq) * grad_scale;
   // a non-finite norm (overflowed fp16 gradients, or a NaN anywhere: fminf would silently drop it) skips the whole update,
   // as GradScaler.step does; torch's clip_grad_norm_ would instead smear the NaN over every parameter
   const bool skip = !(norm <= 3.4028234e38f);
-  const float coef = a.max_norm > 0.f ? fminf(1.f, a.max_norm / (norm + 1e-6f)) * a.grad_scale : a.grad_scale;
+  const float coef = a.max_norm > 0.f ? fminf(1.f, a.max_norm / (norm + 1e-6f)) * grad_scale : grad_scale;
   float bc1 = a.bc1, bc2_sqrt = a.bc2_sqrt;
   if (a.step_dev != nullptr) {  // device-side step count: read by every thread before the last block advances it
     const double t = (double)(*a.step_dev + 1);
@@ -131,6 +139,19 @@ __device__ __forceinline__ void boundary_epilogue(const BoundaryParams& a, float
     if (a.norm_out != nullptr) *a.norm_out = norm;
     if (a.found_inf != nullptr) *a.found_inf = skip ? 1.f : 0.f;
     if (a.step_dev != nullptr && !skip) *a.step_dev += 1;  // every block has read it: this is the last one to finish
+    if (a.amp_scale != nullptr) {  // torch._amp_update_scale_ with found_inf = skip; read by every block, like step_dev
+      const float s = *a.amp_scale;
+      if (skip) {
+        *a.amp_scale = (float)((double)s * a.amp_backoff);
+        *a.amp_tracker = 0;
+      } else if (*a.amp_tracker + 1 == a.amp_interval) {
+        const float grown = (float)((double)s * a.amp_growth);
+        if (isfinite(grown)) *a.amp_scale = grown;  // never grows past the fp32 range
+        *a.amp_tracker = 0;
+      } else {
+        *a.amp_tracker += 1;
+      }
+    }
     a.ws[0] = 0.0;
     *reinterpret_cast<unsigned*>(a.ws + 1) = 0u;
     for (int r = 0; r < a.n_parts; ++r) a.parts[r] = 0.0;  // local copy only: peers zero theirs; next use is behind a barrier
@@ -393,9 +414,11 @@ flat_adamw8_kernel(const __grid_constant__ BoundaryParams h, const __grid_consta
 // ---- host side shared by both entry points (their args structs name the shared fields alike) ---------------------------
 // Validates the shared fields, in the order invalid argument, shape, dtype, alignment, after the entry's own checks
 // `args_ok` (null pointers, tables), `shape_ok` and `aligned` (its 16-byte aligned pointers); launches flat_sumsq_kernel
-// when the norm is needed and was not supplied; fills `b`.  Returns the SM count for the grid clamp, or an error code (< 0).
+// when the norm is needed and was not supplied (always with a loss scaler `sc`, already validated: the norm is its overflow
+// check); fills `b`.  Returns the SM count for the grid clamp, or an error code (< 0).
 template <typename Args>
-int begin_boundary(const Args& o, bool args_ok, bool shape_ok, bool aligned, cudaStream_t st, BoundaryParams& b) {
+int begin_boundary(const Args& o, const psob200_loss_scaler* sc, bool args_ok, bool shape_ok, bool aligned, cudaStream_t st,
+                   BoundaryParams& b) {
   if (!args_ok || !o.param || !o.grad || !o.workspace || o.n <= 0 || (o.step <= 0 && !o.step_dev))
     return PSOB200_ERR_INVALID_ARG;
   if (o.n_sumsq_parts < 0 || (o.n_sumsq_parts > 0 && !o.sumsq_parts)) return PSOB200_ERR_INVALID_ARG;
@@ -404,7 +427,7 @@ int begin_boundary(const Args& o, bool args_ok, bool shape_ok, bool aligned, cud
   if (!aligned) return PSOB200_ERR_ALIGNMENT;
   const int n_sm = sm_count();
   double* ws = reinterpret_cast<double*>(o.workspace);
-  if (o.n_sumsq_parts == 0 && (o.max_grad_norm > 0.f || o.norm_out != nullptr)) {
+  if (o.n_sumsq_parts == 0 && (o.max_grad_norm > 0.f || o.norm_out != nullptr || sc != nullptr)) {
     long long blocks = (o.n + kOptThreads * 4 - 1) / (kOptThreads * 4);
     if (blocks > n_sm * 8) blocks = n_sm * 8;
     flat_sumsq_kernel<<<(unsigned)blocks, kOptThreads, 0, st>>>(o.grad, o.n, ws);
@@ -417,7 +440,19 @@ int begin_boundary(const Args& o, bool args_ok, bool shape_ok, bool aligned, cud
   b.bc2_sqrt = (float)std::sqrt(1.0 - std::pow((double)o.beta2, (double)o.step));
   b.found_inf = o.found_inf; b.step_dev = o.step_dev; b.norm_out = o.norm_out;
   b.ws = ws; b.parts = o.sumsq_parts; b.n_parts = o.n_sumsq_parts;
+  b.amp_scale = sc ? sc->scale : nullptr;
+  b.amp_tracker = sc ? sc->growth_tracker : nullptr;
+  b.amp_growth = sc ? sc->growth_factor : 1.0;
+  b.amp_backoff = sc ? sc->backoff_factor : 1.0;
+  b.amp_interval = sc ? sc->growth_interval : 0;
   return n_sm;
+}
+
+// the optimizer entry points' checks of a loss scaler: both state pointers, a growth that grows, a backoff that shrinks and
+// stays positive, a reachable interval
+inline bool scaler_ok(const psob200_loss_scaler* sc) {
+  return sc != nullptr && sc->scale != nullptr && sc->growth_tracker != nullptr && sc->growth_interval > 0 &&
+         sc->growth_factor > 1.0 && sc->backoff_factor > 0.0 && sc->backoff_factor < 1.0;
 }
 
 // calls f(TO{}) with the element type of the 16-bit operand copy (bf16 when there is none)
@@ -433,12 +468,13 @@ void dispatch_operand(const void* operand, int32_t operand_dtype, F&& f) {
 
 using namespace psob200;
 
-extern "C" int psob200_flat_adamw_step(const psob200_flat_adamw_args* args, void* stream) {
+// sc: a validated loss scaler, or NULL (the unscaled entry points)
+static int flat_adamw_step(const psob200_flat_adamw_args* args, const psob200_loss_scaler* sc, void* stream) {
   if (args == nullptr) return PSOB200_ERR_INVALID_ARG;
   const psob200_flat_adamw_args& o = *args;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   BoundaryParams b;
-  const int n_sm = begin_boundary(o, o.exp_avg && o.exp_avg_sq, true, aligned16(o.grad) && aligned16(o.workspace), st, b);
+  const int n_sm = begin_boundary(o, sc, o.exp_avg && o.exp_avg_sq, true, aligned16(o.grad) && aligned16(o.workspace), st, b);
   if (n_sm < 0) return n_sm;
   long long blocks = (o.n + kOptThreads - 1) / kOptThreads;
   if (blocks > n_sm * 8) blocks = n_sm * 8;
@@ -450,7 +486,17 @@ extern "C" int psob200_flat_adamw_step(const psob200_flat_adamw_args* args, void
   return consume_launch_error("launch flat_adamw_kernel", cudaSuccess);
 }
 
-extern "C" int psob200_flat_adamw8_step(const psob200_flat_adamw8_args* args, void* stream) {
+extern "C" int psob200_flat_adamw_step(const psob200_flat_adamw_args* args, void* stream) {
+  return flat_adamw_step(args, nullptr, stream);
+}
+
+extern "C" int psob200_flat_adamw_step_scaled(const psob200_flat_adamw_args* args, const psob200_loss_scaler* scaler,
+                                              void* stream) {
+  if (!scaler_ok(scaler)) return PSOB200_ERR_INVALID_ARG;
+  return flat_adamw_step(args, scaler, stream);
+}
+
+static int flat_adamw8_step(const psob200_flat_adamw8_args* args, const psob200_loss_scaler* sc, void* stream) {
   if (args == nullptr) return PSOB200_ERR_INVALID_ARG;
   const psob200_flat_adamw8_args& o = *args;
   const bool args_ok =
@@ -463,7 +509,7 @@ extern "C" int psob200_flat_adamw8_step(const psob200_flat_adamw8_args* args, vo
     aligned = aligned && aligned16(p);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   BoundaryParams b;
-  const int n_sm = begin_boundary(o, args_ok, o.block_size == 256 || o.block_size == 2048, aligned, st, b);
+  const int n_sm = begin_boundary(o, sc, args_ok, o.block_size == 256 || o.block_size == 2048, aligned, st, b);
   if (n_sm < 0) return n_sm;
   Adam8State a;
   a.p = o.param; a.g = o.grad; a.c1 = o.code1; a.c2 = o.code2; a.absmax1 = o.absmax1; a.absmax2 = o.absmax2;
@@ -483,6 +529,16 @@ extern "C" int psob200_flat_adamw8_step(const psob200_flat_adamw8_args* args, vo
       flat_adamw8_kernel<256, TO><<<(unsigned)grid, kOpt8Threads, 0, st>>>(b, a, op);
   });
   return consume_launch_error("launch flat_adamw8_kernel", cudaSuccess);
+}
+
+extern "C" int psob200_flat_adamw8_step(const psob200_flat_adamw8_args* args, void* stream) {
+  return flat_adamw8_step(args, nullptr, stream);
+}
+
+extern "C" int psob200_flat_adamw8_step_scaled(const psob200_flat_adamw8_args* args, const psob200_loss_scaler* scaler,
+                                               void* stream) {
+  if (!scaler_ok(scaler)) return PSOB200_ERR_INVALID_ARG;
+  return flat_adamw8_step(args, scaler, stream);
 }
 
 extern "C" int psob200_flat_allreduce_sumsq(const psob200_flat_allreduce_args* args, void* stream) {

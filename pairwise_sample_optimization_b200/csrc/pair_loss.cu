@@ -49,6 +49,7 @@ struct PairKernelArgs {
   int32_t* status;
   unsigned int* counter;
   float* pair_loss;
+  const float* amp_scale;  // device loss scale S (psob200_loss_scaler), NULL = none: multiplies the gradient multipliers
   long long B, N;
   long long stride[4][2];  // element stride between samples: pred, ref, x, xn
   double log_lo, log_hi;   // log(1-eps), log(1+eps): the clamp of T:844-845 expressed on delta
@@ -137,8 +138,14 @@ __device__ __forceinline__ void pair_scalar_function(const PairKernelArgs& a, lo
     st[4] = (float)logits;
     st[5] = (float)per;
   }
-  s_g[0] = (float)g0;
-  s_g[1] = (float)g1;
+  float f0 = (float)g0, f1 = (float)g1;
+  if (a.amp_scale != nullptr) {  // scaled in fp32 after the rounding: a power-of-two S gives exactly S x the unscaled grad
+    const float S = *a.amp_scale;
+    f0 *= S;
+    f1 *= S;
+  }
+  s_g[0] = f0;
+  s_g[1] = f1;
   if (rank == 0) {
     a.pair_loss[pair] = (float)per;
     if (a.stats != nullptr) {
@@ -466,8 +473,9 @@ extern "C" size_t psob200_pair_loss_workspace_bytes(int64_t B) {
   return (size_t)16 + (((size_t)B * sizeof(float) + 15) & ~(size_t)15);
 }
 
-extern "C" int psob200_online_pso_loss_grad(const psob200_schedule* sched, const psob200_online_pso_args* args,
-                                            void* stream) {
+// amp_scale: the device loss scale of a psob200_loss_scaler, or NULL (the unscaled entry points)
+static int online_pso_loss_grad(const psob200_schedule* sched, const psob200_online_pso_args* args, const float* amp_scale,
+                                void* stream) {
   if (sched == nullptr || args == nullptr) return PSOB200_ERR_INVALID_ARG;
   const psob200_online_pso_args& p = *args;
   if (p.B <= 0 || p.N <= 0 || p.loss == nullptr || p.human_prefer == nullptr || p.workspace == nullptr)
@@ -504,6 +512,7 @@ extern "C" int psob200_online_pso_loss_grad(const psob200_schedule* sched, const
   ka.loss = p.loss; ka.stats = p.stats; ka.status = p.status;
   ka.counter = reinterpret_cast<unsigned int*>(p.workspace);
   ka.pair_loss = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(p.workspace) + 16);
+  ka.amp_scale = amp_scale;
   ka.B = p.B; ka.N = p.N; ka.mode = kModeOnline;
   ka.beta = p.beta; ka.eps = p.eps; ka.loss_scale = p.loss_scale;
   const double eps = (double)p.eps;
@@ -513,7 +522,18 @@ extern "C" int psob200_online_pso_loss_grad(const psob200_schedule* sched, const
                      sm_count(), reinterpret_cast<cudaStream_t>(stream));
 }
 
-extern "C" int psob200_dreambooth_pso_loss_grad(const psob200_dreambooth_args* args, void* stream) {
+extern "C" int psob200_online_pso_loss_grad(const psob200_schedule* sched, const psob200_online_pso_args* args,
+                                            void* stream) {
+  return online_pso_loss_grad(sched, args, nullptr, stream);
+}
+
+extern "C" int psob200_online_pso_loss_grad_scaled(const psob200_schedule* sched, const psob200_online_pso_args* args,
+                                                   const psob200_loss_scaler* scaler, void* stream) {
+  if (scaler == nullptr || scaler->scale == nullptr) return PSOB200_ERR_INVALID_ARG;
+  return online_pso_loss_grad(sched, args, scaler->scale, stream);
+}
+
+static int dreambooth_pso_loss_grad(const psob200_dreambooth_args* args, const float* amp_scale, void* stream) {
   if (args == nullptr) return PSOB200_ERR_INVALID_ARG;
   const psob200_dreambooth_args& p = *args;
   if (p.b <= 0 || p.N <= 0 || !p.model_pred || !p.noisy || !p.target || !p.sigmas || !p.grad || !p.loss ||
@@ -543,9 +563,20 @@ extern "C" int psob200_dreambooth_pso_loss_grad(const psob200_dreambooth_args* a
   ka.loss = p.loss; ka.stats = p.stats; ka.status = p.status;
   ka.counter = reinterpret_cast<unsigned int*>(p.workspace);
   ka.pair_loss = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(p.workspace) + 16);
+  ka.amp_scale = amp_scale;
   ka.B = p.b; ka.N = p.N;
   ka.mode = has_ref ? kModeDbPso : kModeDbPsoDb;
   ka.beta = p.beta_pso; ka.nu = p.neg_defactor; ka.lam = p.prior_loss_weight; ka.loss_scale = p.loss_scale;
   return launch_pair(ka, has_ref, p.pred_dtype, p.latent_dtype, vec_ok, p.tune_threads, p.tune_cluster,
                      sm_count(), reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int psob200_dreambooth_pso_loss_grad(const psob200_dreambooth_args* args, void* stream) {
+  return dreambooth_pso_loss_grad(args, nullptr, stream);
+}
+
+extern "C" int psob200_dreambooth_pso_loss_grad_scaled(const psob200_dreambooth_args* args,
+                                                       const psob200_loss_scaler* scaler, void* stream) {
+  if (scaler == nullptr || scaler->scale == nullptr) return PSOB200_ERR_INVALID_ARG;
+  return dreambooth_pso_loss_grad(args, scaler->scale, stream);
 }

@@ -398,6 +398,11 @@ __global__ void __launch_bounds__(V3Cfg<TP, TL, HAS_REF>::kThreads, 1) pair_loss
       }
       float g0, g1, st[8];
       const float per = pair_scalar_function_fast(a, S, ent, g0, g1, st);
+      if (a.amp_scale != nullptr) {  // device loss scale: the gradient is scaled before it is rounded to TP
+        const float amp = *a.amp_scale;
+        g0 *= amp;
+        g1 *= amp;
+      }
       s_g[0] = g0;
       s_g[1] = g1;
       if (rank == 0) {

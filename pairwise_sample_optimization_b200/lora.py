@@ -32,7 +32,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import _lib
+from . import _lib, amp
 
 
 @dataclass
@@ -977,11 +977,15 @@ class FusedLoRAOptimizer:
     ``optim_bits=8`` is the Turbo recipe's ``use_8bit_adam`` (bitsandbytes ``AdamW(optim_bits=8)``, same keyword names):
     blockwise 8-bit moments (``block_size`` elements per fp32 absmax; matrices below ``min_8bit_size`` elements keep fp32
     moments), bitsandbytes' update rule (weight decay after the step), one update launch of psob200_flat_adamw8_step.
-    ``exp_avg`` / ``exp_avg_sq`` are then None; ``dequantized_moments()`` gives flat fp32 copies."""
+    ``exp_avg`` / ``exp_avg_sq`` are then None; ``dequantized_moments()`` gives flat fp32 copies.
+
+    ``grad_scaler`` (an ``amp.DeviceGradScaler``, fp16 training: GradScaler around :857-860): the boundary unscales by
+    ``1 / S`` read on the device (times ``grad_scale``), skips the update on a non-finite norm and updates ``S`` and the
+    growth tracker in the same launch -- ``step()`` stays free of host syncs and capturable in a CUDA graph."""
 
     def __init__(self, model: nn.Module, lr: float = 1e-5, betas=(0.9, 0.999), eps: float = 1e-8,
                  weight_decay: float = 1e-4, max_grad_norm: float = 1.0, exchange: Optional[SymmetricGradExchange] = None,
-                 optim_bits: int = 32, block_size: int = 256, min_8bit_size: int = 4096):
+                 optim_bits: int = 32, block_size: int = 256, min_8bit_size: int = 4096, grad_scaler=None):
         if optim_bits not in (8, 32):
             raise ValueError(f"optim_bits must be 8 or 32, got {optim_bits}")
         if optim_bits == 8 and block_size not in (256, 2048):
@@ -1028,6 +1032,9 @@ class FusedLoRAOptimizer:
         self.found_inf = torch.zeros(1, dtype=torch.float32, device=flat.device)
         self.step_dev = torch.zeros(1, dtype=torch.int64, device=flat.device)  # applied updates (bias correction)
         self.grad_scale = 1.0
+        self.grad_scaler = grad_scaler
+        if grad_scaler is not None:
+            amp.scaler_arg(grad_scaler, flat.device)  # a DeviceGradScaler on this device, or raise now
         self.lr, self.betas, self.eps, self.weight_decay, self.max_grad_norm = lr, betas, eps, weight_decay, max_grad_norm
         self.step_count = 0  # step() calls (host side, no sync); applied updates are counted in `step_dev`
         self._unbacked = []  # adapter matrices whose operand copy needs a padded pitch (rank not a multiple of 8)
@@ -1060,16 +1067,19 @@ class FusedLoRAOptimizer:
     def step(self) -> torch.Tensor:
         """Clip, update, zero the gradient, refresh the operands.  Returns the (pre-clip) gradient norm, on the device."""
         self.step_count += 1
-        entry, a = self._launch_args()
+        entry, a, extra = self._launch_args()
         if self._parts_ready:  # the fused exchange already produced the sum of squares, one piece per rank
             a.n_sumsq_parts, a.sumsq_parts = self.exchange.world, self.exchange.sumsq_parts_ptr
             self._parts_ready = False
-        _lib.launch(self.flat_param.device, entry, C.byref(a), _lib.current_stream(self.flat_param.device))
+        _lib.launch(self.flat_param.device, entry, C.byref(a), *extra, _lib.current_stream(self.flat_param.device))
         self._refresh_unbacked()
         return self.grad_norm
 
     def _launch_args(self):
-        """``(entry point, argument struct)`` of this optimizer's boundary for the next ``step()`` (norm computed in-launch)."""
+        """``(entry point, argument struct, further arguments)`` of this optimizer's boundary for the next ``step()`` (norm
+        computed in-launch); the call is ``entry(byref(struct), *further, stream)``.  With a loss scaler the entry point is
+        the ``_scaled`` one and ``further`` holds the scaler."""
+        extra = ()
         if self.optim_bits == 32:
             entry, a = "psob200_flat_adamw_step", _lib.FlatAdamwArgs()
             a.exp_avg, a.exp_avg_sq = self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr()
@@ -1089,7 +1099,9 @@ class FusedLoRAOptimizer:
         a.lr, a.beta1, a.beta2, a.eps = self.lr, self.betas[0], self.betas[1], self.eps
         a.weight_decay, a.max_grad_norm, a.grad_scale = self.weight_decay, self.max_grad_norm, float(self.grad_scale)
         a.found_inf, a.step_dev = self.found_inf.data_ptr(), self.step_dev.data_ptr()
-        return entry, a
+        if self.grad_scaler is not None:
+            entry, extra = entry + "_scaled", (C.byref(amp.scaler_arg(self.grad_scaler, self.flat_param.device)),)
+        return entry, a, extra
 
     def dequantized_moments(self) -> tuple[torch.Tensor, torch.Tensor]:
         """Flat fp32 copies of both Adam moments in the parameter layout (8-bit blocks dequantised as the kernel does:
@@ -1122,8 +1134,13 @@ class FusedLoRAOptimizer:
         """Everything a resumed run needs for bit-identical continuation: the fp32 master parameters, both Adam moments,
         the count of applied updates (one host sync) and the hyper-parameters.  Tensors are clones on the optimizer's device.
         With ``optim_bits=8`` the moments are the 8-bit state instead (codes, absmax, compact fp32 moments, both maps) and
-        the dict also records ``optim_bits``, ``block_size`` and ``min_8bit_size``."""
+        the dict also records ``optim_bits``, ``block_size`` and ``min_8bit_size``.  With a loss scaler attached it also
+        holds ``scaler_scale`` / ``scaler_growth_tracker`` (the device state) and ``scaler`` (its hyper-parameters)."""
         sd = {k: getattr(self, k).clone() for k in self._state_names}
+        if self.grad_scaler is not None:
+            s = self.grad_scaler
+            sd["scaler_scale"], sd["scaler_growth_tracker"] = s.scale_tensor.clone(), s.growth_tracker.clone()
+            sd["scaler"] = s.hyper()
         sd.update({"step": int(self.step_dev.item()), "step_calls": int(self.step_count),
                    "hyper": {"lr": self.lr, "beta1": self.betas[0], "beta2": self.betas[1], "eps": self.eps,
                              "weight_decay": self.weight_decay, "max_grad_norm": self.max_grad_norm},
@@ -1134,7 +1151,13 @@ class FusedLoRAOptimizer:
 
     def load_state_dict(self, sd: dict, load_hyper: bool = True) -> None:
         """Inverse of ``state_dict()``.  The parameters live in ``flat_param`` (every adapter ``weight`` is a view of it), so
-        loading also restores the adapters; the 16-bit operand copies the GEMM kernels read are refreshed; the gradient is zeroed."""
+        loading also restores the adapters; the 16-bit operand copies the GEMM kernels read are refreshed; the gradient is zeroed.
+        Loss-scaler state loads into the attached scaler (one without such state in ``sd`` keeps its values, as a fresh fp16
+        run would); scaler state with no scaler attached is refused rather than dropped."""
+        has_scaler_state = "scaler_scale" in sd
+        if has_scaler_state and self.grad_scaler is None:
+            raise _lib.Psob200Error("the optimizer state holds loss-scaler state (an fp16 run) but this optimizer has no "
+                                    "grad_scaler: pass grad_scaler=DeviceGradScaler(...) so that it is restored, not dropped")
         bits = int(sd.get("optim_bits", 32))  # fp32 state records no format keys
         if bits != self.optim_bits:
             raise _lib.Psob200Error(f"optimizer state was saved with optim_bits={bits}; this optimizer has optim_bits="
@@ -1156,6 +1179,11 @@ class FusedLoRAOptimizer:
                 getattr(self, k).copy_(sd[k].to(dev))
             self.step_dev.fill_(int(sd["step"]))
             self.flat_operand.copy_(self.flat_param)  # what psob200_flat_adamw_step would have left
+            if has_scaler_state:
+                s = self.grad_scaler
+                s.set_hyper(**sd["scaler"])
+                s.scale_tensor.copy_(sd["scaler_scale"].to(device=s.device, dtype=torch.float32).reshape(1))
+                s.growth_tracker.copy_(sd["scaler_growth_tracker"].to(device=s.device, dtype=torch.int32).reshape(1))
         self.step_count = int(sd.get("step_calls", sd["step"]))
         if load_hyper:
             h = sd["hyper"]

@@ -13,7 +13,7 @@ import ctypes as C
 
 import torch
 
-from . import _lib, runtime
+from . import _lib, amp, runtime
 
 
 # ----------------------------------------------------------------------------- preference signs (a4)
@@ -50,10 +50,21 @@ def _n(t):
     return n
 
 
-def _apply_upstream(grads, grad_out, dev):
-    """d loss was folded into the kernel as 1; scale by autograd's upstream gradient on the device
-    (a no-op launch when it is exactly 1)."""
+def _launch_loss(dev, name, scaler, *args):
+    """The loss launch, through the ``_scaled`` entry point when a ``DeviceGradScaler`` is given."""
+    if scaler is None:
+        _lib.launch(dev, name, *args, _lib.current_stream(dev))
+    else:
+        s = amp.scaler_arg(scaler, dev)
+        _lib.launch(dev, name + "_scaled", *args, C.byref(s), _lib.current_stream(dev))
+
+
+def _apply_upstream(grads, grad_out, dev, scaler=None):
+    """d loss was folded into the kernel as 1 (as S with a loss scaler); scale by autograd's upstream gradient (divided by
+    S) on the device -- a no-op launch when that is exactly 1, e.g. after ``scaler.scale(loss).backward()``."""
     go = grad_out.detach().reshape(1).to(torch.float32)
+    if scaler is not None:
+        go = go / scaler.scale_tensor
     for g in grads:
         _lib.launch(dev, "psob200_scale_inplace_by_device_scalar", g.data_ptr(), g.numel(), _lib.dtype_code(g),
                                                                go.data_ptr(), _lib.current_stream(dev))
@@ -62,7 +73,7 @@ def _apply_upstream(grads, grad_out, dev):
 class _OnlinePsoLoss(torch.autograd.Function):
     @staticmethod
     def forward(ctx, pred0, pred1, ref0, ref1, x0, x1, xn0, xn1, ts0, ts1, tsp0, tsp1, coef0, coef1, h, sched,
-                beta, eps, loss_scale, want_stats, tune):
+                beta, eps, loss_scale, want_stats, tune, scaler):
         dev = _lib.require_cuda(pred0, pred1, ref0, ref1, x0, x1, xn0, xn1, h)
         B, n = pred0.shape[0], _n(pred0)
         a = _lib.OnlinePsoArgs()
@@ -103,9 +114,10 @@ class _OnlinePsoLoss(torch.autograd.Function):
         a.pred_dtype, a.latent_dtype = _lib.dtype_code(pred0), _lib.dtype_code(keep[2])
         a.beta, a.eps, a.loss_scale = float(beta), float(eps), float(loss_scale)
         a.tune_threads, a.tune_cluster = tune
-        _lib.launch(dev, "psob200_online_pso_loss_grad", sched.ref(), C.byref(a), _lib.current_stream(dev))
+        _launch_loss(dev, "psob200_online_pso_loss_grad", scaler, sched.ref(), C.byref(a))
         ctx.save_for_backward(grad0, grad1)
         ctx.dev = dev
+        ctx.scaler = scaler
         ctx.used = False
         if stats is not None:
             ctx.mark_non_differentiable(stats)
@@ -118,13 +130,13 @@ class _OnlinePsoLoss(torch.autograd.Function):
             raise RuntimeError("pso_pair_loss: backward may run only once (its gradient buffers are consumed)")
         ctx.used = True
         grad0, grad1 = ctx.saved_tensors
-        _apply_upstream((grad0, grad1), grad_loss, ctx.dev)
-        return (grad0, grad1) + (None,) * 19
+        _apply_upstream((grad0, grad1), grad_loss, ctx.dev, ctx.scaler)
+        return (grad0, grad1) + (None,) * 20
 
 
 def pso_pair_loss(noise_pred_0, noise_pred_1, noise_ref_pred_0, noise_ref_pred_1, sample_0, sample_1, next_0, next_1,
                   timesteps_0, timesteps_1, human_prefer, *, scheduler=None, kind="turbo", beta=50.0, eps=0.1,
-                  step_ratio=None, coefficients=None, loss_scale=1.0, return_stats=False, tune=(0, 0)):
+                  step_ratio=None, coefficients=None, loss_scale=1.0, return_stats=False, tune=(0, 0), grad_scaler=None):
     """Online PSO loss of one micro-step, differentiable w.r.t. ``noise_pred_0/1`` only.
 
     kind="turbo": ``scheduler.timesteps/.sigmas`` are read (EulerAncestral; T:810-837);
@@ -134,6 +146,10 @@ def pso_pair_loss(noise_pred_0, noise_pred_1, noise_ref_pred_0, noise_ref_pred_1
     ``loss_scale`` folds accelerate's ``loss / gradient_accumulation_steps`` (T:857) into the
     same launch.  Returns ``loss`` (0-dim fp32) or ``(loss, stats[B,8])`` with
     stats = (logp_pol0, logp_ref0, logp_pol1, logp_ref1, delta0, delta1, z, pair_loss).
+    ``grad_scaler`` (an ``amp.DeviceGradScaler``, fp16 training): the kernel computes the gradient already multiplied by
+    the device scale S, so it is rounded to the prediction dtype scaled; the backward divides autograd's upstream factor
+    by S, so ``grad_scaler.scale(loss).backward()`` leaves S x the gradient and ``loss.backward()`` the unscaled one.
+    ``loss`` and ``stats`` are unscaled either way.
     """
     dev = _lib.require_cuda(noise_pred_0)
     ts0 = ts1 = tsp0 = tsp1 = c0 = c1 = None
@@ -159,7 +175,7 @@ def pso_pair_loss(noise_pred_0, noise_pred_1, noise_ref_pred_0, noise_ref_pred_1
     loss, stats = _OnlinePsoLoss.apply(noise_pred_0, noise_pred_1, noise_ref_pred_0.detach(), noise_ref_pred_1.detach(),
                                        sample_0.detach(), sample_1.detach(), next_0.detach(), next_1.detach(),
                                        ts0, ts1, tsp0, tsp1, c0, c1, human_prefer, sched, beta, eps, loss_scale,
-                                       return_stats, tune)
+                                       return_stats, tune, grad_scaler)
     return (loss, stats) if return_stats else loss
 
 
@@ -182,7 +198,7 @@ def edm_sigmas(noise_scheduler, timesteps: torch.Tensor, n_dim: int = 4, dtype=t
 class _DreamboothPsoLoss(torch.autograd.Function):
     @staticmethod
     def forward(ctx, model_pred, ref_pred, noisy, target, sigmas, loss_type, beta_pso, neg_defactor,
-                prior_loss_weight, loss_scale, tune):
+                prior_loss_weight, loss_scale, tune, scaler):
         dev = _lib.require_cuda(model_pred, ref_pred, noisy, target, sigmas)
         b2, n = model_pred.shape[0], _n(model_pred)
         if b2 % 2:
@@ -212,10 +228,11 @@ class _DreamboothPsoLoss(torch.autograd.Function):
         a.beta_pso, a.neg_defactor = float(beta_pso), float(neg_defactor)
         a.prior_loss_weight, a.loss_scale = float(prior_loss_weight), float(loss_scale)
         a.tune_threads, a.tune_cluster = tune
-        _lib.launch(dev, "psob200_dreambooth_pso_loss_grad", C.byref(a), _lib.current_stream(dev))
+        _launch_loss(dev, "psob200_dreambooth_pso_loss_grad", scaler, C.byref(a))
         del rp, tg, sg
         ctx.save_for_backward(grad)
         ctx.dev = dev
+        ctx.scaler = scaler
         ctx.used = False
         ctx.mark_non_differentiable(stats)
         return loss, stats
@@ -226,12 +243,12 @@ class _DreamboothPsoLoss(torch.autograd.Function):
             raise RuntimeError("pso_db_loss: backward may run only once (its gradient buffer is consumed)")
         ctx.used = True
         (grad,) = ctx.saved_tensors
-        _apply_upstream((grad,), grad_loss, ctx.dev)
-        return (grad,) + (None,) * 10
+        _apply_upstream((grad,), grad_loss, ctx.dev, ctx.scaler)
+        return (grad,) + (None,) * 11
 
 
 def pso_db_loss(model_pred, ref_pred, noisy_model_input, model_input, sigmas, *, loss_type="pso", beta_pso=1.0,
-                neg_defactor=0.1, prior_loss_weight=0.0, loss_scale=1.0, tune=(0, 0)):
+                neg_defactor=0.1, prior_loss_weight=0.0, loss_scale=1.0, tune=(0, 0), grad_scaler=None):
     """DreamBooth-PSO loss (train_pso_sdxl_turbo_dreambooth.py:1847-1865,1881-1935) on RAW UNet
     outputs: the EDM-style epsilon preconditioning ``x0_hat = -sigma*pred + noisy`` (:1855), the
     ``sigma^-2`` weighting (:1865), the win/lose chunking (:1891), the optional reference branch
@@ -239,7 +256,7 @@ def pso_db_loss(model_pred, ref_pred, noisy_model_input, model_input, sigmas, *,
 
     Returns ``(loss, model_losses_w[b], model_losses_l[b], logits[b])`` -- the three extras feed the
     logging at :1941-1950 and carry no gradient.  ``loss_type`` is "pso" or "pso_db"; anything else
-    raises ValueError like :1929.
+    raises ValueError like :1929.  ``grad_scaler``: as in ``pso_pair_loss`` (fp16 loss scaling, :1953 under GradScaler).
     """
     if loss_type == "pso":
         lt = _lib.DB_PSO
@@ -251,5 +268,5 @@ def pso_db_loss(model_pred, ref_pred, noisy_model_input, model_input, sigmas, *,
         raise ValueError(f"Unknown loss type {loss_type}")
     loss, stats = _DreamboothPsoLoss.apply(model_pred, None if ref_pred is None else ref_pred.detach(),
                                            noisy_model_input.detach(), model_input.detach(), sigmas, lt, beta_pso,
-                                           neg_defactor, prior_loss_weight, loss_scale, tune)
+                                           neg_defactor, prior_loss_weight, loss_scale, tune, grad_scaler)
     return loss, stats[:, 0], stats[:, 1], stats[:, 4]
