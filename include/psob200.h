@@ -676,6 +676,79 @@ PSOB200_API int psob200_geglu_forward(const psob200_geglu_args* args, void* stre
 PSOB200_API int psob200_geglu_backward(const psob200_geglu_args* args, void* stream);
 
 /*
+ * LayerNorm over the last dimension (torch.nn.LayerNorm with one normalised dimension: the norm1 / norm2 / norm3 of every
+ * diffusers==0.27.0 BasicTransformerBlock), forward and backward, one launch each.  Not a row of the PSO hot path
+ * (SURVEY.md section 8): the stock norm kernels were the largest stock item after the attention core.
+ *   x [rows, C] of dtype (row pitch ld_x); weight / bias [C] of param_dtype, each may be NULL (1 resp. 0).
+ *   forward:  y = (x - mean) rstd weight + bias   [rows, C] of out_dtype;  mean, rstd: float[rows]
+ *             mean = sum x / C,  rstd = 1 / sqrt(sum (x - mean)^2 / C + eps)   (fp32, centred two-pass)
+ *   backward: dx = rstd (g - mean_C g - xhat mean_C(g xhat)),  g = dy weight,  xhat = (x - mean) rstd   (dy of out_dtype,
+ *             dx of dtype; no weight / bias gradient: the base model is frozen)
+ * dtype F32 / BF16 / F16; out_dtype = dtype, or F32 (autocast: layer_norm runs in fp32 on 16-bit input).  C a multiple of 8,
+ * at most 2048; row pitches multiples of 8 elements; x, y, dy, dx 16-byte aligned.  Deterministic.
+ */
+typedef struct psob200_layer_norm_args {
+  const void* x;
+  void* y;
+  const void* dy;
+  void* dx;
+  const void* weight;
+  const void* bias;
+  float* mean;
+  float* rstd;
+  int64_t rows, C;
+  int64_t ld_x, ld_y, ld_dy, ld_dx;
+  float eps;
+  int32_t dtype;
+  int32_t out_dtype;
+  int32_t param_dtype;
+} psob200_layer_norm_args;
+
+PSOB200_API int psob200_layer_norm_forward(const psob200_layer_norm_args* args, void* stream);
+PSOB200_API int psob200_layer_norm_backward(const psob200_layer_norm_args* args, void* stream);
+
+/*
+ * GroupNorm over contiguous NCHW (torch.nn.GroupNorm), optionally fused with what surrounds it in diffusers==0.27.0
+ * ResnetBlock2D.forward: `nonlinearity(norm1(x))` (silu != 0) and `nonlinearity(norm2(h + time_emb_proj(temb)[:, :, None,
+ * None]))` (silu != 0 and channel_add = the [N, C] projection).  Forward and backward, two launches each.
+ *   x [N, C, HW] of dtype; channel_add [N, C] of dtype or NULL: xs = round_to_dtype(x + channel_add[n, c]) is what is
+ *   normalised (the stock add's rounding; the backward recomputes it); weight / bias [C] of param_dtype or NULL.
+ *   Group g of sample n = channels [g C / G, (g + 1) C / G), one contiguous span of S = (C / G) HW elements.
+ *   forward:  z = (xs - mean) rstd weight[c] + bias[c];  y = silu ? z sigmoid(z) : z   ([N, C, HW] of out_dtype)
+ *             mean, rstd: float[N G] (biased variance, Chan's pairwise merge of per-part moments)
+ *   backward: g = dy (silu ? silu'(z) : 1) weight[c];  dx = rstd (g - mean_S g - xhat mean_S(g xhat))   (dx of dtype; no
+ *             weight / bias / channel_add gradient: the base model is frozen)
+ * Any HW >= 1 and any C divisible by G (else PSOB200_ERR_SHAPE).  workspace: >= psob200_group_norm_workspace_bytes(N, C, HW,
+ * G) bytes, 16-byte aligned, no initialisation needed (cross-CTA partials of one call; one workspace per stream).
+ * x, y, dy, dx 16-byte aligned.  dtype / out_dtype as psob200_layer_norm_args.  Deterministic: every group is cut into parts
+ * that depend on the shape only, and the parts are combined in a fixed order.
+ */
+typedef struct psob200_group_norm_args {
+  const void* x;
+  const void* channel_add;
+  void* y;
+  const void* dy;
+  void* dx;
+  const void* weight;
+  const void* bias;
+  float* mean;
+  float* rstd;
+  void* workspace;
+  size_t workspace_bytes;
+  int64_t N, C, HW;
+  int32_t G;
+  float eps;
+  int32_t dtype;
+  int32_t out_dtype;
+  int32_t param_dtype;
+  int32_t silu;
+} psob200_group_norm_args;
+
+PSOB200_API size_t psob200_group_norm_workspace_bytes(int64_t N, int64_t C, int64_t HW, int32_t G);
+PSOB200_API int psob200_group_norm_forward(const psob200_group_norm_args* args, void* stream);
+PSOB200_API int psob200_group_norm_backward(const psob200_group_norm_args* args, void* stream);
+
+/*
  * Reward-side image preprocessing on the device (SURVEY.md section 8f rank 4).  Replaces, in one launch, the round trip the
  * trainers make before every reward call (train_online_pso_sdxl_turbo.py:632-640, pso_pytorch/pickscore_utils.py:24-33):
  *     ((images + 1) * 127.5).clamp(0, 255).to(uint8).permute(0,2,3,1).cpu().numpy() -> PIL.Image.fromarray -> CLIPImageProcessor
@@ -719,7 +792,8 @@ PSOB200_API int psob200_clip_preprocess(const psob200_clip_preprocess_args* args
  * 2 dreambooth_args, 3 step_args, 4 step_bwd_args, 5 gemm_args,
  * 6 lora_linear_args, 7 flat_adamw_args, 8 geglu_args,
  * 9 flat_allreduce_args, 10 clip_preprocess_args, 11 lora_group_args,
- * 12 flat_adamw8_args, 13 loss_scaler.  Returns 0 for unknown ids. */
+ * 12 flat_adamw8_args, 13 loss_scaler, 14 layer_norm_args, 15 group_norm_args.
+ * Returns 0 for unknown ids. */
 PSOB200_API size_t psob200_struct_size(int which);
 
 #ifdef __cplusplus

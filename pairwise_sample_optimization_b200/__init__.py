@@ -7,6 +7,7 @@ Only what the path needs (SURVEY.md section 8):
 * ``losses``                      fused online-PSO and DreamBooth-PSO loss + gradient
 * ``lora`` / ``gemm``              LoRA-wrapped attention projections (peft / diffusers surface) on the tcgen05 GEMM kernels
 * ``feed_forward``                fused gated GELU (GEGLU) of the transformer feed-forward, forward + backward
+* ``norms``                       fused LayerNorm / GroupNorm (+ SiLU, + the ResNet time-embedding add), forward + backward
 * ``checkpoint``                  LoRA adapters in the reference's safetensors wire format (+ optimizer state)
 * ``reward_preprocess``           decoded images -> CLIP / PickScore ``pixel_values`` on the device (Pillow-exact resize)
 * ``runtime``                     device-resident schedule tables, workspace, status word
@@ -14,7 +15,7 @@ Only what the path needs (SURVEY.md section 8):
 
 There is no CPU or PyTorch fallback: every op raises if the CUDA library is missing.
 """
-from . import _lib, amp, checkpoint, feed_forward, gemm, lora, reward_preprocess, runtime
+from . import _lib, amp, checkpoint, feed_forward, gemm, lora, norms, reward_preprocess, runtime
 from .amp import DeviceGradScaler
 from .losses import compare, edm_sigmas, pso_db_loss, pso_pair_loss, sample_compare
 from .pso_pytorch.diffusers_patch import (

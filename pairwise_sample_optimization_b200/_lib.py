@@ -144,9 +144,23 @@ class ClipPreprocessArgs(C.Structure):
                 ("dst_dtype", C.c_int32)]
 
 
+class LayerNormArgs(C.Structure):
+    _fields_ = [("x", _vp), ("y", _vp), ("dy", _vp), ("dx", _vp), ("weight", _vp), ("bias", _vp), ("mean", _fp), ("rstd", _fp),
+                ("rows", C.c_int64), ("C", C.c_int64), ("ld_x", C.c_int64), ("ld_y", C.c_int64), ("ld_dy", C.c_int64),
+                ("ld_dx", C.c_int64), ("eps", C.c_float), ("dtype", C.c_int32), ("out_dtype", C.c_int32),
+                ("param_dtype", C.c_int32)]
+
+
+class GroupNormArgs(C.Structure):
+    _fields_ = [("x", _vp), ("channel_add", _vp), ("y", _vp), ("dy", _vp), ("dx", _vp), ("weight", _vp), ("bias", _vp),
+                ("mean", _fp), ("rstd", _fp), ("workspace", _vp), ("workspace_bytes", C.c_size_t), ("N", C.c_int64),
+                ("C", C.c_int64), ("HW", C.c_int64), ("G", C.c_int32), ("eps", C.c_float), ("dtype", C.c_int32),
+                ("out_dtype", C.c_int32), ("param_dtype", C.c_int32), ("silu", C.c_int32)]
+
+
 _STRUCTS = {0: Schedule, 1: OnlinePsoArgs, 2: DreamboothArgs, 3: StepArgs, 4: StepBwdArgs, 5: GemmArgs,
             6: LoraLinearArgs, 7: FlatAdamwArgs, 8: GegluArgs, 9: FlatAllreduceArgs, 10: ClipPreprocessArgs, 11: LoraGroupArgs,
-            12: FlatAdamw8Args, 13: LossScaler}
+            12: FlatAdamw8Args, 13: LossScaler, 14: LayerNormArgs, 15: GroupNormArgs}
 
 # name -> (restype, argtypes): every symbol include/psob200.h declares
 SIGNATURES = {
@@ -179,6 +193,11 @@ SIGNATURES = {
     "psob200_flat_allreduce_sumsq": (C.c_int, [C.POINTER(FlatAllreduceArgs), _vp]),
     "psob200_geglu_forward": (C.c_int, [C.POINTER(GegluArgs), _vp]),
     "psob200_geglu_backward": (C.c_int, [C.POINTER(GegluArgs), _vp]),
+    "psob200_layer_norm_forward": (C.c_int, [C.POINTER(LayerNormArgs), _vp]),
+    "psob200_layer_norm_backward": (C.c_int, [C.POINTER(LayerNormArgs), _vp]),
+    "psob200_group_norm_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int64, C.c_int64, C.c_int32]),
+    "psob200_group_norm_forward": (C.c_int, [C.POINTER(GroupNormArgs), _vp]),
+    "psob200_group_norm_backward": (C.c_int, [C.POINTER(GroupNormArgs), _vp]),
     "psob200_resample_taps": (C.c_int, [C.c_int64, C.c_int64]),
     "psob200_resample_plan": (C.c_int, [C.c_int64, C.c_int64, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "psob200_clip_norm_table": (C.c_int, [C.c_double, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float)]),

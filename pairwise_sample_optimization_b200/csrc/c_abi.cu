@@ -58,6 +58,8 @@ extern "C" size_t psob200_struct_size(int which) {
     case 11: return sizeof(psob200_lora_group_args);
     case 12: return sizeof(psob200_flat_adamw8_args);
     case 13: return sizeof(psob200_loss_scaler);
+    case 14: return sizeof(psob200_layer_norm_args);
+    case 15: return sizeof(psob200_group_norm_args);
     default: return 0;
   }
 }

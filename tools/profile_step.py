@@ -17,6 +17,7 @@ ap.add_argument("--pairs", type=int, default=4)
 ap.add_argument("--top", type=int, default=40)
 ap.add_argument("--grad-checkpointing", action="store_true")
 ap.add_argument("--no-fused-geglu", action="store_true")
+ap.add_argument("--fused-norms", action="store_true", help="LayerNorm / GroupNorm (+ SiLU) on the fused kernels (norms.install_fused_norms)")
 args = ap.parse_args()
 conf = bench.CONFIGS[args.config]
 dev = torch.device("cuda", 0)
@@ -34,6 +35,9 @@ if args.grad_checkpointing:
 if not args.no_fused_geglu:
     from pairwise_sample_optimization_b200 import feed_forward
     feed_forward.install_fused_geglu(unet)
+if args.fused_norms:
+    from pairwise_sample_optimization_b200 import norms
+    norms.install_fused_norms(unet)
 bucket = lora.LoRAGradBucket(lora.lora_parameters(unet))
 sched = bench.turbo_scheduler() if conf["kind"] == "turbo" else bench.dmd_scheduler()
 host = micro_step.batched_view(micro_step.synth_batch(args.pairs, conf["latent_hw"], 2048, 1280, 100, getattr(sched, "sigmas", None),
